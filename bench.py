@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (torchrun for N > 1)
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle port)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write what the last timed step computed (.npy)
 
 A "step" is ONE EPISODE of the batched env: reset (row sampling, user-history GRU-1 + input
 projections) followed by max_steps x env.step (act, feature assembly, DIEN forward, reward/done),
@@ -222,6 +223,28 @@ def workload_config(args, seq):
                   "exceeds the 126 MB L2; no explicit flush"}
 
 
+DUMP_ROWS = 512                                                 # --dump-outputs: env rows kept of the [T, B, ...] arrays
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(dirname, arrays, batch, row_axis):
+    """Write what the last timed step handed its caller as DIR/<name>.npy (float32, or float64 where float32 would round),
+    keeping a fixed, seeded sample of DUMP_ROWS env rows (axis `row_axis`) of the arrays that hold a feature vector per
+    row, so that two builds can be compared."""
+    rows = np.sort(np.random.RandomState(0).choice(batch, min(batch, DUMP_ROWS), replace=False))
+    out = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        if a.ndim > row_axis + 1 and a.shape[row_axis] == batch:
+            a = np.take(a, rows, axis=row_axis)
+        out[name] = a.astype(np.float64 if a.dtype.itemsize > 4 or a.dtype.kind in "iu" else np.float32)
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_LIMIT, "outputs to dump: %d bytes" % total
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def emit(line):
     """The ONE JSON line goes to the real stdout; everything else (NCCL's version banner, library
     chatter) was redirected to stderr at start-up so the driver can parse stdout."""
@@ -237,7 +260,7 @@ if __name__ == "__main__":                      # not when imported (tests, the 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--env", default="slate", choices=["slate", "seqslate"])
@@ -250,7 +273,11 @@ def main():
     ap.add_argument("--cpu-sample-rows", type=int, default=128, help="CPU arm: at most this many env rows per worker process")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--kernels", action="store_true", help="also print a per-kernel time breakdown (stderr)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (rank 0; at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     world_env = int(os.environ.get("WORLD_SIZE", "1"))
     if world_env > 1:
         args.gpus = world_env
@@ -307,14 +334,21 @@ def main():
                 a = env.offline_action                                  # logged items' embeddings, f64 [B, 32] on the device
                 a = a + 0.3 * torch.randn(a.shape, generator=gen, device=dev, dtype=a.dtype)
                 obs, reward, done, info = env.step(a)
-            return reward
+            return {"obs": obs["obs"], "action_mask": obs["action_mask"], "reward": reward, "done": done}
 
         episode_device = episode_env_only = rollout_conti
     else:
         trainer = (PPOTrainer({"sgd_minibatch_size": args.sgd_minibatch}, env, seed=0) if args.algo == "ppo"
                    else A2CTrainer({}, env, seed=0))                     # modelfree_train.py:179-217 / :248-304
         learner_launches = lambda: trainer.ops.launches
-        episode_device = trainer.train                                   # rollout + learner pass
+
+        def episode_device():                                            # rollout + learner pass
+            stats = trainer.train()
+            b = trainer.buf
+            out = {"obs": b.obs, "action_mask": b.mask, "action": b.action, "logp": b.logp, "value": b.value,
+                   "logits": b.logits, "reward": b.reward, "policy_params": trainer.policy.flat}
+            out.update({"stats_" + k: np.float64(v) for k, v in stats.items() if isinstance(v, (int, float))})
+            return out
         episode_env_only = lambda: trainer.rollout(explore=True)
 
     def barrier():
@@ -327,13 +361,13 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     for _ in range(args.warmup):
         episode_device()
@@ -342,13 +376,15 @@ def main():
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()
-    ms = timed(episode_device, args.steps)
+    ms, last = timed(episode_device, args.steps)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, B, row_axis=0 if args.conti else 1)
     prof = eng.profile_read()
     eng.profile(0)
     gpu_launches = eng.launch_count() + learner_launches() - launches0   # env kernels + policy/learner kernels
     value = B * world * T * args.steps / (ms / 1e3)
-    ms_env = timed(episode_env_only, args.steps)
+    ms_env, _ = timed(episode_env_only, args.steps)
     env_only = B * world * T * args.steps / (ms_env / 1e3)
 
     # ---- e2e: reference-facing call, host buffers (README.md:14-21 loop) ------------------------
@@ -364,7 +400,7 @@ def main():
 
     for _ in range(args.warmup):
         episode_host()
-    ms_h = timed(episode_host, args.steps)
+    ms_h, _ = timed(episode_host, args.steps)
     e2e = B * world * T * args.steps / (ms_h / 1e3)
     act_bytes = B * 32 * 8 if args.conti else B * 4
     h2d = B * 4 + T * act_bytes

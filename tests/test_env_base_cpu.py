@@ -1,10 +1,14 @@
 """CPU: the gym layer (rl4rs_b200.env.base.RecEnvBase / build_spaces) over a fake simulator, held against the
-reference's OWN RecEnvBase (rl4rs/env/base.py:178-273, run through oracle/ref_harness.py) when /root/reference is
-present, and against the recorded expectations otherwise."""
+reference's OWN RecEnvBase (rl4rs/env/base.py:178-273, run through oracle/ref_harness.py over the same fake simulator;
+what it showed is stored in tests/golden/reference/expected.json by tests/golden/make_reference_golden.py)."""
+import hashlib
+import json
+import os
+
 import numpy as np
 import pytest
 
-from oracle import ref_harness
+from golden_util import REFERENCE_DIR
 from rl4rs_b200.env.base import RecEnvBase, build_spaces
 
 A, OBS = 284, 256
@@ -119,11 +123,14 @@ def test_env_layer_matches_reference_env_layer(name, batch):
         assert [c[1] for c in ours["calls"] if c[0] == "step"] == [[7], [7]]        # a bare action is wrapped
     else:
         assert ours["user"] == [200, 201, 202] and ours["r1"][1] == [1.0, 2.0, 3.0]
-    if not ref_harness.reference_available():
-        pytest.skip("reference tree absent: recorded expectations only")
-    ref_base = ref_harness.install_stubs()[0]
-    ref = drive(ref_base.RecEnvBase, config)
-    assert ref == ours
+    with open(os.path.join(REFERENCE_DIR, "expected.json")) as f:
+        ref = json.load(f)["env_layer"]["%s/%d" % (name, batch)]
+    assert seen_digest(ours) == ref, ours
+
+
+def seen_digest(seen):
+    """What drive() saw, as a digest of its JSON form (tuples become lists)."""
+    return hashlib.sha256(json.dumps(seen, sort_keys=True).encode()).hexdigest()
 
 
 def test_build_spaces_takes_the_widths_from_the_config():

@@ -1,7 +1,7 @@
 """CPU: the simulator graphs as the REFERENCE'S OWN code wires them (rl4rs/nets/*.py run through oracle/tf_eager_stub.py,
-vectors committed by tests/golden/make_nets_golden.py) against (i) the NumPy oracles the GPU tests compare with and
-(ii) the variable-scope plans of the TF1 checkpoint reader.  Pins wiring and scope order, not the third-party layer
-arithmetic (see the stub's header)."""
+vectors committed by tests/golden/make_nets_golden.py and tests/golden/make_reference_golden.py) against (i) the NumPy
+oracles the GPU tests compare with and (ii) the variable-scope plans of the TF1 checkpoint reader.  Pins wiring and scope
+order, not the third-party layer arithmetic (see the stub's header)."""
 import json
 import os
 import sys
@@ -12,8 +12,7 @@ import pytest
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
 import make_nets_golden as mk                                   # noqa: E402
 
-from golden_util import golden_names                            # noqa: E402
-from oracle import ref_harness                                  # noqa: E402
+from golden_util import REFERENCE_DIR, check_fingerprint, digest, golden_names, load_fingerprint   # noqa: E402
 from oracle.dien_np import DienOracle                           # noqa: E402
 from oracle.dnn_np import DnnOracle                             # noqa: E402
 from oracle.lstm_np import LstmOracle                           # noqa: E402
@@ -21,6 +20,7 @@ from oracle.widedeep_np import WideDeepOracle                   # noqa: E402
 from rl4rs_b200.utils import tf_checkpoint as tfc               # noqa: E402
 
 ORACLES = {"dien": DienOracle, "dnn": DnnOracle, "widedeep": WideDeepOracle, "lstm": LstmOracle}
+RECORDS = os.path.join(REFERENCE_DIR, "records.npz")
 PLANS = {"dien": tfc.dien_layer_plan, "dnn": tfc.dnn_layer_plan, "widedeep": tfc.widedeep_layer_plan, "lstm": tfc.lstm_layer_plan}
 
 
@@ -69,29 +69,35 @@ def test_checkpoint_plan_follows_the_reference_creation_order(golden, case):
 
 
 def test_checkpoint_file_feeds_the_reference_graph(golden, tmp_path):
-    """n1 end to end: W-table -> Saver-format bundle on disk -> TensorBundleReader -> the reference's graph code."""
-    if not ref_harness.reference_available():
-        pytest.skip("reference tree absent")
-    from oracle import tf_eager_stub as stub
-    g, _ = golden
+    """n1 end to end: W-table -> Saver-format bundle on disk -> TensorBundleReader -> the reference's graph code.  The
+    reference's graph turned the tensors read back from the file into dien_stress_obs; the committed digest of those
+    tensors (tests/golden/make_reference_golden.py) holds today's writer and reader to them."""
     w, _ = mk.checkpoint_of("dien_stress")
     rd = tfc.TensorBundleReader(tfc.save_dien_checkpoint(str(tmp_path / "sim"), w, mk.SMALL))
     ck = {name: rd.get_tensor(name) for name in rd.variables()}
-    r = stub.run_reference_graph("dien", mk.NETS_CONFIG, ck, g["seq"].astype(np.float32), g["dense"], g["cat"])
-    assert not r["unused"]
-    np.testing.assert_array_equal(r["obs"], g["dien_stress_obs"])
+    want = expected_nets()["checkpoint_file_tensors"]
+    assert sorted(ck) == sorted(want)
+    for name in sorted(ck):
+        assert digest(ck[name]) == want[name], name
 
 
 @pytest.mark.parametrize("case", sorted(mk.CASES))
 def test_committed_vectors_are_what_the_reference_code_computes_now(golden, case):
-    if not ref_harness.reference_available():
-        pytest.skip("reference tree absent")
-    from oracle import tf_eager_stub as stub
+    """The vectors were computed by the reference's graph from mk.checkpoint_of(case) and the committed feature rows;
+    tests/golden/make_reference_golden.py re-ran that graph, found the vectors and scopes unchanged, and stored a digest
+    of each checkpoint tensor.  Today's checkpoint_of must still give those tensors."""
     g, meta = golden
     _, ck = mk.checkpoint_of(case)
-    r = stub.run_reference_graph(mk.CASES[case][0], mk.NETS_CONFIG, ck, g["seq"].astype(np.float32), g["dense"], g["cat"])
-    np.testing.assert_allclose(r["obs"], g[case + "_obs"], rtol=0, atol=1e-13 * max(1.0, np.abs(r["obs"]).max()))
-    assert [[s, n, list(sh)] for s, n, sh in r["variables"]] == meta[case]["variables"] and r["layers"] == meta[case]["layers"]
+    want = expected_nets()["checkpoints"][case]
+    assert sorted(ck) == sorted(want)
+    for name in sorted(ck):
+        assert digest(ck[name]) == want[name], (case, name)
+    assert sorted(n for _, n, _ in meta[case]["variables"]) == sorted(ck)
+
+
+def expected_nets():
+    with open(os.path.join(REFERENCE_DIR, "expected.json")) as f:
+        return json.load(f)["nets"]
 
 
 def test_the_check_has_teeth(golden):
@@ -109,45 +115,32 @@ def test_the_references_own_stack_reproduces_the_fixtures(name):
     reference builds ITSELF -- RecEnvBase -> (Seq)SlateRecEnv.__init__ -> RecSimBase.__init__ -> rl4rs/nets/dien.py ->
     tf.train.Saver().restore of a checkpoint written by our n1 writer -> keras.backend.function -> obs_fn / forward --
     over the layer stand-ins, replays the fixture's actions, and must land on the fixture: integers exactly, observations
-    and rewards at f32 rounding (the stand-ins compute in f64 and hand back float32 like keras.backend.function)."""
-    if not ref_harness.reference_available():
-        pytest.skip("reference tree absent")
-    sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-    import make_golden
+    and rewards at f32 rounding (the stand-ins compute in f64 and hand back float32 like keras.backend.function).  What
+    that stack recorded is stored in tests/golden/reference/records.npz (tests/golden/make_reference_golden.py)."""
     from golden_util import Golden
     g = Golden(name)
-    a = g.arr
-    T = g.config["max_steps"]
-    replay = lambda env, ep, t, off: a["action_in"][ep * T + t]
-    rec = make_golden.run_reference(g.config, g.meta["records"], g.meta["catalog_text"], g.weights, g.seq, replay,
-                                    n_episodes=g.n_episodes, seed=g.meta.get("np_seed"), full_stack=True)
-    assert set(rec) == set(a), set(rec) ^ set(a)
-    for key in sorted(a):
-        if key in ("reset_obs", "step_obs", "reward", "click_p"):
-            ref = a[key].astype(np.float64)
-            if key.endswith("obs") and ref.shape[-1] > 256:              # d3rl form: obs | masked_actions | cur_steps
-                np.testing.assert_array_equal(rec[key][..., 256:], ref[..., 256:], err_msg=key)
-                got, ref = rec[key][..., :256], ref[..., :256]
-            else:
-                got = rec[key]
-            scale = np.maximum(np.abs(ref), np.sqrt((ref ** 2).mean(axis=-1, keepdims=True)) if ref.ndim > 1 else 1.0)
-            assert (np.abs(got - ref) / np.maximum(scale, 1e-6)).max() < 3e-5, key
-        elif a[key].dtype.kind == "f":
-            np.testing.assert_allclose(rec[key], a[key], rtol=1e-12, atol=0, err_msg=key)
-        else:
-            np.testing.assert_array_equal(rec[key], a[key], err_msg=key)
+    check_fingerprint(g.arr, load_fingerprint(RECORDS, "fixture_stack/" + name), rtol=3e-5, what=name + " (full stack)")
 
 
 @pytest.mark.parametrize("algo,seq", [("dnn", False), ("widedeep", True), ("lstm", False)])
 def test_the_references_own_stack_with_the_other_simulators(algo, seq):
     """config['algo'] dispatch (slate.py:239-242) through the reference's own constructors for the other three graphs of
     rl4rs/nets/: a short logged-policy episode of the self-constructed reference env against the oracle env the GPU tests
-    use for that simulator (tests/test_gpu_dnn.py)."""
-    if not ref_harness.reference_available():
-        pytest.skip("reference tree absent")
-    sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-    import make_golden
+    use for that simulator (tests/test_gpu_dnn.py).  What the reference recorded is stored in
+    tests/golden/reference/records.npz (tests/golden/make_reference_golden.py)."""
     from oracle.env_np import OracleEnv
+    from rl4rs_b200.utils.datautil import FeatureUtil
+    from test_oracle_vs_reference_random import roll_oracle
+    cfg, cat, records, w = other_simulator_inputs(algo, seq)
+    ora = OracleEnv(cfg, FeatureUtil.parse_log(records, 64), cat, ORACLES[algo](w, np.float32), seq=seq)
+    rec = roll_oracle(ora, cfg, lambda env, ep, t, off: off, 1)
+    check_fingerprint(rec, load_fingerprint(RECORDS, "simulator/" + algo), rtol=3e-5, what="%s simulator" % algo)
+    assert rec["step_obs"].shape[-1] == (3072 if algo == "widedeep" else 256) and (rec["reward"] > 0).any()
+
+
+def other_simulator_inputs(algo, seq):
+    """(cfg, catalog, log records, weights) of the short logged-policy episode for simulator `algo`."""
+    import make_golden
     from rl4rs_b200 import synth
     B = 4
     cfg = dict(make_golden.BASE_CFG, batch_size=B, cache_size=B, is_eval=True, support_rllib_mask=True, algo=algo,
@@ -156,30 +149,36 @@ def test_the_references_own_stack_with_the_other_simulators(algo, seq):
     log = synth.make_log(12, pages=4 if seq else 1, catalog=cat, hash_size=600, keep_hist=True)
     records = synth.render_records(log, cat)
     maker = {"dnn": synth.make_dnn_weights, "widedeep": synth.make_widedeep_weights, "lstm": synth.make_lstm_weights}[algo]
-    w = maker(cfg, stress=2.0, bias_noise=0.2)
-    rec = make_golden.run_reference(cfg, records, cat.to_text(), w, seq, lambda env, ep, t, off: off, full_stack=True)
-    from rl4rs_b200.utils.datautil import FeatureUtil
-    ora = OracleEnv(cfg, FeatureUtil.parse_log(records, 64), cat, ORACLES[algo](w, np.float32), seq=seq)
-    obs = ora.reset()
-    np.testing.assert_allclose(rec["reset_obs"][0], obs["obs"], rtol=0, atol=3e-5 * max(1.0, np.abs(obs["obs"]).max()))
-    for t in range(cfg["max_steps"]):
-        np.testing.assert_array_equal(rec["offline_action"][t], ora.offline_action)
-        obs, reward, done, _ = ora.step(ora.offline_action)
-        np.testing.assert_array_equal(rec["step_action_mask"][t], obs["action_mask"])
-        np.testing.assert_allclose(rec["step_obs"][t], obs["obs"], rtol=0, atol=3e-5 * max(1.0, np.abs(obs["obs"]).max()))
-        np.testing.assert_allclose(rec["reward"][t], reward, rtol=3e-5, atol=1e-9)
-        np.testing.assert_array_equal(rec["done"][t], done)
-    assert rec["step_obs"].shape[-1] == (3072 if algo == "widedeep" else 256) and (rec["reward"] > 0).any()
+    return cfg, cat, records, maker(cfg, stress=2.0, bias_noise=0.2)
 
 
 def test_rllib_policy_models_of_the_reference_against_the_torch_twins():
     """a22 / n4: rl4rs/nets/rllib/rllib_rawstate_model.py's TFModelWithRawState (its own Keras graph over nets/utils.py)
     and rllib_mask_model.py's MyMaskActionsModel.forward (the action masking), run from the reference tree over the
-    stand-ins, against rl4rs_b200/policy.py -- the twins the kernels k_policy_act / k_policy_grad are themselves held to."""
-    if not ref_harness.reference_available():
-        pytest.skip("reference tree absent")
+    stand-ins, against rl4rs_b200/policy.py -- the twins the kernels k_policy_act / k_policy_grad are themselves held to.
+    What the reference's models returned is stored in tests/golden/reference/records.npz
+    (tests/golden/make_reference_golden.py)."""
+    c = rllib_case()
+    z = np.load(RECORDS)
+    out = {k[len("rllib/"):]: z[k] for k in z.files if k.startswith("rllib/")}
+    scopes = [str(x) for x in out["scopes"]]
+    assert not out["unused"].size
+    assert [s_ for i, s_ in enumerate(scopes) if i == 0 or s_ != scopes[i - 1]] == \
+        ["embedding", "dense", "dense_1", "embedding_1", "dense_2", "fc_out", "value_out"]       # Keras creation order
+    np.testing.assert_allclose(out["logits"], c["logits"].numpy(), rtol=0, atol=2e-5)
+    np.testing.assert_allclose(out["value"], c["value"].numpy(), rtol=0, atol=2e-5)
+    # the masking itself, by the reference's forward(): fed the twin's unmasked logits as the action_embed_model output
+    np.testing.assert_array_equal(out["masked"], c["masked"].numpy())
+    # and for the 256-d observation policy of the benchmark configs
+    got = out["masked256"]
+    np.testing.assert_array_equal(got, c["want256"].numpy())
+    assert (got[c["mask"] == 0] < -1e38).all()
+
+
+def rllib_case():
+    """The raw-state policy twin with perturbed weights, its checkpoint under the reference model's scope names, six
+    random raw-state rows and action masks, and what the twins compute on them."""
     import torch
-    from oracle import tf_eager_stub as stub
     from rl4rs_b200.policy import MaskedPolicy, RawStatePolicy
     cfg = {"category_hash_size": 600, "emb_size": 128, "hidden_units": 128, "category_feature_num": 21,
            "dense_feature_num": 432, "seq_num": 2, "maxlen": 64, "batch_size": 6}
@@ -196,26 +195,14 @@ def test_rllib_policy_models_of_the_reference_against_the_torch_twins():
           "dense_1/bias": p["db2"], "embedding_1/embeddings": p["emb_seq"], "dense_2/kernel": p["wc"], "dense_2/bias": p["bc"],
           "fc_out/kernel": p["w2"], "fc_out/bias": p["b2"], "value_out/kernel": p["wv"], "value_out/bias": p["bv"]}
     cat, dense, seq = rs.randint(0, 600, (R, 21)), rs.normal(0, 2, (R, 432)).astype(np.float32), rs.randint(0, 284, (R, 2, 64))
-    out = stub.run_reference_rawstate_model(cfg, ck, cat.astype(np.float32), dense, seq.astype(np.float32), A)
-    scopes = [v[0] for v in out["variables"]]
-    assert not out["unused"]
-    assert [s_ for i, s_ in enumerate(scopes) if i == 0 or s_ != scopes[i - 1]] == \
-        ["embedding", "dense", "dense_1", "embedding_1", "dense_2", "fc_out", "value_out"]       # Keras creation order
     obs = pol.pack({"category_feature": torch.as_tensor(cat), "dense_feature": torch.as_tensor(dense), "sequence_feature": torch.as_tensor(seq)})
     with torch.no_grad():
         logits, value = pol.forward(obs, torch.ones(R, A))
         masked, _ = pol.forward(obs, torch.as_tensor(mask))
-    np.testing.assert_allclose(out["logits"], logits.numpy(), rtol=0, atol=2e-5)
-    np.testing.assert_allclose(out["value"], value.numpy(), rtol=0, atol=2e-5)
-    # the masking itself, by the reference's forward(): fed the twin's unmasked logits as the action_embed_model output
-    got = stub.run_reference_mask_forward(lambda o: logits.numpy(), obs.numpy(), mask, A)
-    np.testing.assert_array_equal(got, masked.numpy())
-    # and for the 256-d observation policy of the benchmark configs
     mp = MaskedPolicy(A, "cpu", seed=5)
     o256 = torch.as_tensor(rs.normal(0, 1, (R, 256)).astype(np.float32))
     with torch.no_grad():
         raw, _ = mp.forward(o256, torch.ones(R, A))
-        want, _ = mp.forward(o256, torch.as_tensor(mask))
-    got = stub.run_reference_mask_forward(lambda o: raw.numpy(), o256.numpy(), mask, A)
-    np.testing.assert_array_equal(got, want.numpy())
-    assert (got[mask == 0] < -1e38).all()
+        want256, _ = mp.forward(o256, torch.as_tensor(mask))
+    return {"cfg": cfg, "A": A, "mask": mask, "ck": ck, "cat": cat, "dense": dense, "seq": seq, "obs": obs,
+            "logits": logits, "value": value, "masked": masked, "o256": o256, "raw": raw, "want256": want256}
