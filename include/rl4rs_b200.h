@@ -171,21 +171,15 @@ int r4_augru_kernel_for(int ctas, int sms);
 /* Process-wide kernel-choice overrides for parity tests and A/B timing (no reference counterpart):
  *   "augru_kernel"     0 = by r4_augru_kernel_for (default), 2 = always the pair kernel, 3 = always the ping-pong pair kernel
  *                      (two recurrences per pair)
- *   "augru_pair_impl"  hand-over / weight-ring variant of the pair kernels, <RELAY, TMAP>: 1 = <0,0> (default: direct
- *                      release.cta arrive, per-CTA bulk-copy ring), 2 = <0,1> (tensor-map ring), 3 = <1,0> (relayed
- *                      release.cluster hand-over), 4 = <1,1>
  *   "augru_cost_pair" / "augru_cost_pp"  the per-wave costs r4_augru_kernel_for compares (positive ints)
- *   "augru_cluster"    CTAs per cluster of the pair kernel: 2 (one pair), 4 or 8 (2 / 4 pairs share one multicast weight stream)
  *   "pay_obs_reuse"    1 (default): r4_step takes the observation of a PAYING step (the last step of a slate / page) from that
  *                      step's reward pass -- the state the step leaves (rl4rs/env/slate.py:203-213, seqslate.py:104-122) is the
  *                      last of the page's complete states (slate.py:117-131, seqslate.py:27-50), so the reference runs the same
  *                      feature row through the simulator twice; 0: launch the separate observation pass as well
- *   "scores_impl"      DIN attention scores (nets/utils.py:121-122): 2 (default) = k_scores_tc2, both attention layers on the
- *                      tensor pipe with the second GEMM's A operand in tensor memory; 1 = k_scores_tc (second layer as FMAs)
  *   "scores_shared_pct" share of an even CTA split given to a sequence whose cached rows are shared by all feature rows
  *                      (Slate's constant second sequence), 10..100 per cent
- * The environment variables R4_AUGRU_PAIR / R4_AUGRU_PP / R4_AUGRU_PAIR_IMPL / R4_AUGRU_RULE / R4_NO_PAY_OBS_REUSE / R4_SCORES_IMPL give the initial
- * values.  Returns 0, or R4_ERR_ARG for an unknown key / out-of-range value. */
+ * The environment variables R4_AUGRU_PAIR / R4_AUGRU_PP / R4_AUGRU_RULE / R4_NO_PAY_OBS_REUSE give the initial values.
+ * Returns 0, or R4_ERR_ARG for an unknown key / out-of-range value. */
 int r4_set_option(const char* key, int value);
 
 /* ---- policy + learner (K12): MyMaskActionsModel (rllib_mask_model.py:41-62) and the RLlib PPO / A2C losses ----

@@ -1,9 +1,26 @@
-// r4_augru_pair2.cuh -- second generation of the 2-CTA AUGRU recurrence (deepctr VecAttGRUCell, nets/utils.py:123-124).
-// Same arithmetic, TMEM / shared-memory layout and weight image as k_augru_pair (r4_augru_pair.cuh); what changed is
-// everything around the tensor pipe, each item answering a measurement of round 1:
+// r4_augru_pair2.cuh -- the AUGRU recurrence (deepctr VecAttGRUCell, nets/utils.py:123-124) as ONE tensor-core instruction
+// stream per 2-CTA cluster: tcgen05.mma.cta_group::2, M = 128 (64 feature rows per CTA), N = 256, bf16 hi/lo operands, fp32
+// accumulators in both CTAs' TMEM.  The arithmetic (r4_tc_common.cuh):
+//     r = sigmoid(Xr_t + h Wr)      u = sigmoid(Xu_t + h Wu)      c = tanh(Xc_t + (r*h) Wc)
+//     u' = (1 - score_t) u ;  h <- u' h + (1 - u') c              (3 bf16 products per fp32 product)
+// What the pair buys (measured with tools/pair_probe.cu): a 128x256x16 MMA takes 64 cycles instead of 128, each CTA streams
+// only its half of the weight columns, each CTA's epilogue owns 64 rows instead of 128 (so a 4096-row batch x 2 sequences
+// fills 128 SMs instead of 64), and the accumulators of one gate take 128 TMEM columns per CTA -- r, u and c do not alias,
+// and r*h gets its own A buffer, so the gate epilogues overlap the next gate's MMAs.
+// TMEM layout of a pair MMA (cute tmem_frg_2sm "2x2" atom, confirmed by the probe): in each CTA, lanes 0-63 hold
+// accumulator columns 0-127 of the CTA's 64 rows and lanes 64-127 hold columns 128-255.
+//
+// Per CTA: shared memory = A(h) hi/lo 64 KB + A(r*h) hi/lo 64 KB + a 3-stage ring of 16 KB weight stages (one 32-deep K
+// block of the CTA's 128 weight columns, hi then lo split, pre-tiled on the host so a stage is one bulk copy).  Both CTAs'
+// stages must have landed before the leader issues: the peer's control warp relays its local "full" barrier to the leader
+// with a remote mbarrier arrive (~460 cycles one way, hidden by the ring).
+// Warp roles: 0-7 epilogue (TMEM lane quarter q = warp & 3, column half = warp >> 2; thread = one row x 64 hidden
+// columns), 8 = MMA issuer (leader) / ring relay (peer), 9 = TMA producer, 10-11 idle.
+//
+// Around the tensor pipe, each item answering a measurement of round 1:
 //   * issue loop: the whole MMA warp walks the step in uniform control flow, ONE lane elected once (elect.sync) issues,
-//     ring stage / mbarrier parity / operand offsets are compile-time constants (a step = 24 ring uses = 4 revolutions
-//     of the 6 stages, so they repeat every step).  Round 1: ~100 SASS instructions of descriptor arithmetic + an
+//     ring stage / mbarrier parity / operand offsets are compile-time constants (a step = 24 ring uses = 8 revolutions
+//     of the 3 stages, so they repeat every step).  Round 1: ~100 SASS instructions of descriptor arithmetic + an
 //     ELECT/BRA.U.ANY wrapper per MMA paced the pair MMAs at ~105 cycles; this form issues at 52-65.
 //   * rolling input prefetch: the epilogue keeps the inputs of the NEXT gate phase in registers (x[4][16]); a chunk is
 //     reloaded with the next phase's columns the moment it has been consumed, so every L2 load has a whole phase
@@ -13,40 +30,92 @@
 //     fence.proxy.async -> __syncwarp -> one mbarrier.arrive.release.cta on the LEADER's barrier (a shared::cluster address
 //     for the peer: the instruction CUTLASS's ClusterBarrier::arrive(cta_id) issues for the peer-epilogue -> leader-MMA
 //     signals of its 2-SM kernels).  The data a peer warp publishes stays in the PEER's shared memory and is read by the
-//     peer SM's half of the cta_group::2 MMA; what crosses the cluster is only the arrival.  Round 1 used a .relaxed remote
-//     arrive (advisor finding: not a release); .release.cluster on the arriving warps costs 2x the kernel (30 k cycles per
-//     step: ~320 cycles per arrive, 8 per step and warp, on the critical path of the chasing MMAs).  RELAY = 1 keeps the
-//     strictly cluster-scoped chain as an option: the peer's warps arrive on a barrier in their OWN CTA and one relay lane
-//     per operand (warps 10 / 11 of the peer) forwards each completed quarter with mbarrier.arrive.release.cluster --
-//     19.3 k cycles per step against 15.5 k.
-//   * weight ring by tensor-map TMA (TMAP = 1, optional; the per-CTA bulk-copy ring measured faster): both CTAs issue cp.async.bulk.tensor.2d.cta_group::2 for
-//     their own half of the stage with the LEADER's "full" barrier as the completion target, the leader's producer
-//     posts one expect_tx for both halves.  No relay thread, no remote arrive: the transaction count is the signal.
-//     The image is viewed as a 2-D tensor of 1 KB rows, a stage is a 256 x 16 box of u32 (16 KB, dense).
+//     peer SM's half of the cta_group::2 MMA; what crosses the cluster is only the arrival.
+// Measured alternatives (tools/augru_probe.cu, round 2, cycles per step; DESIGN.md section 4): a relayed release.cluster
+// hand-over 19.3 k and a tensor-map weight ring 17.2 k, against 15.5 k for this kernel.
 #pragma once
 #include <cuda.h>
-#include "r4_augru_pair.cuh"
-
-// Defaults of the product build (r4_capi.cu: augru_pair_impl 1), chosen by measurement (tools/augru_probe.cu, round 2, 64
-// tiles, cycles per step): <RELAY 0, TMAP 0> 15.5 k | <0,1> 17.2 k | <1,1> 19.3 k.
-#ifndef R4P2_RELAY
-#define R4P2_RELAY 0
-#endif
-#ifndef R4P2_TMAP
-#define R4P2_TMAP 0
-#endif
-#ifndef R4P2_PRESCALE
-#define R4P2_PRESCALE 0   // 1: the cached input halves arrive pre-multiplied (r, u columns by -log2(e), c columns by 2 log2(e)),
-#endif                    //    so a gate pre-activation in the exp2 domain is ONE fma(acc, scale, x') instead of add + mul
-#ifndef R4P2_SWPIPE
-#define R4P2_SWPIPE 0     // 1: the bf16 split + shared-memory store of chunk k-1 is issued next to the MUFU section of chunk k
-#endif
+#include "r4_tc_common.cuh"
 
 namespace r4tc {
 
+constexpr int P_RC = 64;                              // rows per CTA
+constexpr int P_NB = 128;                             // weight columns (B rows) per CTA
+constexpr int P_HALF_BYTES = P_NB * KB * 2;           // 8192: one split of one 32-deep K block of the CTA's 128 columns
+constexpr int P_STAGE_BYTES = 2 * P_HALF_BYTES;       // 16384: ring stage = [hi | lo] of one K block (6 MMAs, 384 cycles)
+constexpr int P_STAGES_PER_STEP = 3 * NKB;            // 24
+// Ring depth.  Measured (tools/augru_probe.cu, round 2, cycles per step of k_augru_pair2 / k_augru_pp): 6 stages 17.1 k /
+// 31.3 k, 4 stages 16.0 k / 31.4 k, 3 stages 15.7 k / 29.6 k, 2 stages 20.5 k.  A deep ring refills in bursts that compete
+// with the gate epilogues for the shared-memory port (the MMA warp's own clocks: with 6 stages it waits 7-8 k cycles per
+// step for operand quarters, i.e. for the epilogue, with 3 stages 2.7 k); 3 stages = 48 KB keeps the weight stream just
+// ahead of the MMAs.  24 % (2 * P_NST) == 0 keeps stage and parity compile-time.
+constexpr int P_NST = 3;
+constexpr int P_A_BYTES = P_RC * HID * 2;             // 32768 per split
+constexpr int P_SMEM_BYTES = 4 * P_A_BYTES + P_NST * P_STAGE_BYTES + 128;
+constexpr int P_RANK_IMAGE_BYTES = P_STAGES_PER_STEP * P_STAGE_BYTES; // 393216 per CTA rank
+constexpr int P_TC_R = 0, P_TC_U = 128, P_TC_C = 256;                  // TMEM column bases of the gates
+
+__device__ __forceinline__ void mma2_bf16(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t acc) {
+  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+               "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
+               :: "r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(acc) : "memory");
+}
+// completion of all earlier MMAs of this thread -> one arrival on the barrier at this offset in BOTH CTAs
+__device__ __forceinline__ void commit2(uint64_t* bar) {
+  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+               :: "r"(smem_u32(bar)), "h"((uint16_t)3) : "memory");
+}
+// acquire.cluster try_wait is expensive (a producer loop built on it issued one stage per ~450 cycles); it is used
+// only for the barriers the leader's MMA thread waits on, which collect remote arrivals.
+__device__ __forceinline__ void mbar_wait_cl(uint64_t* bar, uint32_t parity) {
+  asm volatile("{\n\t.reg .pred p;\n\tWAIT_LOOP:\n\t"
+               "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1;\n\t"
+               "@p bra DONE;\n\tbra WAIT_LOOP;\n\tDONE:\n\t}\n" :: "r"(smem_u32(bar)), "r"(parity) : "memory");
+}
+__device__ __forceinline__ uint32_t mapa_rank(uint32_t laddr, uint32_t rank) {
+  uint32_t r; asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(laddr), "r"(rank)); return r;
+}
+// Arrival on a barrier of the other CTA of the pair: mbarrier.arrive.release.cta (the default semantics of
+// mbarrier.arrive: CUTLASS's ClusterBarrier::arrive(cta_id)).  It is enough where the data being published lives in the
+// ARRIVING CTA's own shared memory and has already been made visible to the async proxy (TMA completion, or
+// fence.proxy.async by every writer + __syncwarp): the consumer is this SM's tensor core, started by the leader only after
+// it has observed the arrival.  Measured (cycles per step): .relaxed.cluster 15.5 k, .release.cta 15.5 k, .release.cluster
+// 30.1 k (it blocks its thread ~320 cycles, tools/pair_probe.cu).
+__device__ __forceinline__ void arrive_remote(uint32_t caddr) {
+  asm volatile("mbarrier.arrive.release.cta.shared::cluster.b64 _, [%0];" :: "r"(caddr) : "memory");
+}
+__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
+__device__ __forceinline__ void cluster_sync_all() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+
+// Ring stage s8 (0..7) of every gate holds K block 0,4,1,5,2,6,3,7: the epilogue of k_augru_pair2 completes the blocks
+// {q, 4 + q} of an A operand with its q-th column chunk, and the MMAs follow it in that order.
+__host__ __device__ constexpr int pair_kb(int s8) { return (s8 & 1) * 4 + (s8 >> 1); }
+
+// host: fp32 recurrent weights -> [rank 2][mat r,u,c][8 K blocks][hi, lo] stages of 128 columns x 32 K (8 KB).
+// Wg: [256][512] rows = h index, columns [r | u];  Wc: [256][256].
+inline void build_pair_image(const float* Wg, const float* Wc, uint8_t* img) {
+  for (int rank = 0; rank < 2; ++rank)
+    for (int mat = 0; mat < 3; ++mat)
+      for (int kb = 0; kb < NKB; ++kb)
+        for (int sp = 0; sp < 2; ++sp) {
+          const int kbsrc = pair_kb(kb);               // the order in which the kernels walk the K blocks of a gate
+          uint8_t* st = img + (size_t)rank * P_RANK_IMAGE_BYTES + (size_t)((mat * NKB + kb) * 2 + sp) * P_HALF_BYTES;
+          for (int nl = 0; nl < P_NB; ++nl)
+            for (int kk = 0; kk < KB; ++kk) {
+              const int k = kbsrc * KB + kk, n = rank * P_NB + nl;
+              float w = mat == 0 ? Wg[(size_t)k * 2 * HID + n] : (mat == 1 ? Wg[(size_t)k * 2 * HID + HID + n] : Wc[(size_t)k * HID + n]);
+              uint16_t hi = host_bf16_bits(w);
+              uint16_t v = sp == 0 ? hi : host_bf16_bits(w - host_bf16_val(hi));
+              memcpy(st + (nl / 8) * B_SBO + (kk / 8) * LBO + (nl % 8) * 16 + (kk % 8) * 2, &v, 2);
+            }
+        }
+}
+
 struct AugruPairParams {
   AugruTcParams b;
-  CUtensorMap tmap[2];        // per sequence: the pair weight image as [rows of 1 KB][256 x u32] (TMAP variants only)
+  CUtensorMap tmap[2];        // per sequence: the pair weight image as [rows of 1 KB][256 x u32] (k_augru_pp's weight ring)
 };
 
 // Descriptor of a SWIZZLE_NONE K-major operand split into its two words: `lo` carries the start address (>> 4, 14 bits)
@@ -56,34 +125,11 @@ __device__ __forceinline__ uint32_t desc_lo(uint32_t saddr, uint32_t lbo) { retu
 __device__ __forceinline__ constexpr uint32_t desc_hi(uint32_t sbo) { return ((sbo >> 4) & 0x3fffu) | (1u << 14); }
 __device__ __forceinline__ uint64_t desc_of(uint32_t lo, uint32_t hi) { return ((uint64_t)hi << 32) | lo; }
 
-__device__ __forceinline__ uint32_t elect_one() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .b32 r;\n\t.reg .pred p;\n\telect.sync r|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}\n" : "=r"(pred));
-  return pred;
-}
-
-// this CTA's 16 KB box of the weight image -> own shared memory, completion bytes -> the barrier at `mbar_cluster`
-// (a shared::cluster address: the leader's "full" barrier for both CTAs of the pair)
-__device__ __forceinline__ void tma_box_cg2(uint32_t dst_smem, const CUtensorMap* tm, int c0, int c1, uint32_t mbar_cluster) {
-  asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-               :: "r"(dst_smem), "l"(reinterpret_cast<uint64_t>(tm)), "r"(c0), "r"(c1), "r"(mbar_cluster) : "memory");
-}
-
-// the same, MULTICAST: one L2 read delivers the box to the same shared-memory offset of every CTA in `mask`; with
-// cta_group::2 each destination's completion bytes go to the barrier of ITS pair's even CTA (the operand names the
-// even-CTA position of the issuer's pair).  This is what lets several CTA pairs of a cluster share one weight stream.
-__device__ __forceinline__ void tma_box_cg2_mc(uint32_t dst_smem, const CUtensorMap* tm, int c0, int c1, uint32_t mbar_cluster, uint16_t mask) {
-  asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%2, %3}], [%4], %5;"
-               :: "r"(dst_smem), "l"(reinterpret_cast<uint64_t>(tm)), "r"(c0), "r"(c1), "r"(mbar_cluster), "h"(mask) : "memory");
-}
 // tcgen05.commit -> one arrival on the barrier at this offset in every CTA of `mask`
 __device__ __forceinline__ void commit2_mask(uint64_t* bar, uint16_t mask) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
                :: "r"(smem_u32(bar)), "h"(mask) : "memory");
 }
-
-constexpr int P2_TM_ROW_BYTES = 1024;                             // tensor-map row = 256 x u32
-constexpr int P2_TM_BOX_ROWS = P_STAGE_BYTES / P2_TM_ROW_BYTES;   // 16 rows per ring stage
 
 // One gate of one step: 8 ring stages x 2 K16 slices x (A_hi*B_hi + A_lo*B_hi + A_hi*B_lo).  Every gate walks the K
 // blocks of its A operand in the order pair_kb() = 0,4,1,5,2,6,3,7: the epilogue finishes blocks {q, 4 + q} with its
@@ -93,7 +139,7 @@ constexpr int P2_TM_BOX_ROWS = P_STAGE_BYTES / P2_TM_ROW_BYTES;   // 16 rows per
 template <int GATE>
 __device__ __forceinline__ void issue_gate2(uint32_t leader, uint32_t tbase, uint32_t aHi_lo, uint32_t aLo_lo, uint32_t b_lo,
                                             uint64_t* bar_full, uint64_t* bar_empty, uint64_t* qbar, uint32_t qpar,
-                                            uint16_t empty_mask = 3, long long* wait_acc = nullptr) {
+                                            long long* wait_acc = nullptr) {
   constexpr uint32_t idesc = make_idesc(TM, HID);
   constexpr uint32_t dcol = GATE == 0 ? P_TC_R : (GATE == 1 ? P_TC_U : P_TC_C);
   constexpr uint32_t a_hi = desc_hi(A_SBO), b_hi = desc_hi(B_SBO);
@@ -120,81 +166,23 @@ __device__ __forceinline__ void issue_gate2(uint32_t leader, uint32_t tbase, uin
         mma2_bf16(tbase + dcol, dal, dbh, idesc, 1u);
         mma2_bf16(tbase + dcol, dah, dbl, idesc, 1u);
       }
-      commit2_mask(&bar_empty[stage], empty_mask);
+      commit2(&bar_empty[stage]);
     }
     __syncwarp();
   }
 }
 
-#ifndef R4_ABL
-#define R4_ABL 0          // ABLATION PROBES ONLY (results become wrong): 1 no bf16 split + st.shared, 2 no tcgen05.ld/st in the
-#endif                    // epilogue, 4 no global input loads, 8 no MUFU -- which part of a gate phase costs what (tools/augru_probe.cu)
-#ifndef R4_SOFTRCP
-#define R4_SOFTRCP 0      // reciprocals of the gate epilogues on the FMA pipe: 0 none (all MUFU.RCP), 1 all, 2 every second element
-#endif
-// 1 / x for 1 <= x < 2^122 without the MUFU pipe: exponent-flip seed (5 % error), one cubic step e + e^2 and one Newton
-// step -- 5 FMAs + 1 integer subtract, relative error <= 1.2e-7 (1 ulp class, like rcp.approx).  The gate epilogues need
-// 5 MUFU operations per state element (3 ex2 + 2 rcp) and are bound by that pipe (16 results / clk / SM); moving the
-// reciprocals to the FMA pipe (128 lanes / clk / SM) trades 1 MUFU slot for 6 issue slots.
-__device__ __forceinline__ float soft_rcp(float x) {
-  float y = __int_as_float(0x7EF311C7 - __float_as_int(x));
-  float e = fmaf(-x, y, 1.0f);
-  y = fmaf(y, fmaf(e, e, e), y);
-  e = fmaf(-x, y, 1.0f);
-  return fmaf(y, e, y);
-}
-// reciprocal of element j of a chunk: the pipe is a compile-time choice per element
-__device__ __forceinline__ float rcp_sel(float x, int j) {
-  return (R4_SOFTRCP == 1 || (R4_SOFTRCP == 2 && (j & 1))) ? soft_rcp(x) : rcp_approx(x);
-}
-constexpr float P2_NL2E = -1.4426950408889634f, P2_2L2E = 2.8853900817779268f;
-// gate pre-activation in the exp2 domain: scale * (acc + x); with R4P2_PRESCALE x already carries the scale
-__device__ __forceinline__ float preact2(float acc, float x, float scale) {
-#if R4P2_PRESCALE
-  return fmaf(acc, scale, x);
-#else
-  return scale * (acc + x);
-#endif
-}
+constexpr float P2_NL2E = -1.4426950408889634f, P2_2L2E = 2.8853900817779268f;   // gate pre-activations in the exp2 domain
 // 8 fp32 -> bf16 hi / lo core-matrix rows of an A operand
 __device__ __forceinline__ void split_store8(const float* v, uint8_t* hi_base, uint8_t* lo_base, uint32_t off) {
-#if R4_ABL & 1
-  if (v[0] == 1234.5678f) *reinterpret_cast<float*>(hi_base + off) = v[1];     // keeps the values live, never taken
-#else
   uint4 hi, lo;
   split8(v, hi, lo);
   *reinterpret_cast<uint4*>(hi_base + off) = hi;
   *reinterpret_cast<uint4*>(lo_base + off) = lo;
-#endif
 }
-#if R4_ABL & 2
-#define P2_TMEM_LD16(addr, dst) do { _Pragma("unroll") for (int q_ = 0; q_ < 16; ++q_) (dst)[q_] = 0.25f; } while (0)
-#define P2_TMEM_ST16(addr, src) do { if ((src)[0] == 1234.5678f) asm volatile("" :: "f"((src)[1])); } while (0)
-#define P2_TMEM_WAIT_LD() do { } while (0)
-#define P2_TMEM_WAIT_ST() do { } while (0)
-#else
-#define P2_TMEM_LD16(addr, dst) tmem_ld16((addr), (dst))
-#define P2_TMEM_ST16(addr, src) tmem_st16((addr), (src))
-#define P2_TMEM_WAIT_LD() tmem_wait_ld()
-#define P2_TMEM_WAIT_ST() tmem_wait_st()
-#endif
-#if R4_ABL & 8
-__device__ __forceinline__ float p2_ex2(float x) { return x * 0.001f + 1.0f; }
-__device__ __forceinline__ float p2_rcp(float x, int) { return 2.0f - x * 0.5f; }
-#else
-__device__ __forceinline__ float p2_ex2(float x) { return ex2_approx(x); }
-__device__ __forceinline__ float p2_rcp(float x, int j) { return rcp_sel(x, j); }
-#endif
 
-// CS = CTAs per cluster (2, 4 or 8; set at launch with cudaLaunchAttributeClusterDimension): CS / 2 CTA pairs working on
-// consecutive row tiles of the SAME sequence share ONE weight stream -- pair 0's producers multicast every ring stage to
-// all pairs.  Why: chip-wide the recurrence is bound by L2 throughput, not by the tensor pipe (ablation probes, round 2:
-// 128 CTAs x (393 KB weights + 196 KB inputs) per step = 75 MB against ~6300 B/clk of L2 -> 12 k cycles; without the
-// input loads 13.6 k, without any epilogue work 11.4 k of the 17.3 k-cycle step).  Sharing the stream between 2 (4)
-// pairs cuts the weight traffic to 1/2 (1/4).  Requires TMAP.
-template <int RELAY, int TMAP, int CS = 2>
+// Launched in clusters of 2 CTAs (cudaLaunchAttributeClusterDimension): one CTA pair per 128-row tile and sequence.
 __global__ void __launch_bounds__(NTHREADS, 1) k_augru_pair2(const __grid_constant__ AugruPairParams pp) {
-  static_assert(CS == 2 || TMAP, "weight-stream sharing needs the tensor-map ring");
   extern __shared__ uint8_t smem_raw[];
   __shared__ uint64_t bar_full[P_NST], bar_empty[P_NST], bar_h[4], bar_rh[4], bar_r, bar_u, bar_c;
   __shared__ uint32_t tmem_base_s;
@@ -207,23 +195,22 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_augru_pair2(const __grid_consta
   uint8_t* sB = smem + 4 * P_A_BYTES;
   const AugruTcSeq& S = p.s[blockIdx.y];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const uint32_t crank = cluster_ctarank();    // rank in the cluster: pair = crank >> 1
+  // The leader's cluster rank and the tile are derived for a general cluster shape although a cluster is one pair here
+  // (lead = 0, every pair has a tile): written as constants, they reorder the machine code of the whole kernel.
+  const uint32_t crank = cluster_ctarank();
   const uint32_t rank = crank & 1;             // rank inside the CTA pair: 0 = leader (issues the MMAs)
   const uint32_t lead = crank & ~1u;           // cluster rank of this pair's leader
   const int n_tiles = (p.R + TM - 1) / TM;
-  const int tile = min((int)(blockIdx.x >> 1), n_tiles - 1);   // padding pairs of the last cluster redo the last tile, unseen
-  const bool pad_pair = (int)(blockIdx.x >> 1) >= n_tiles;
+  const int tile = min((int)(blockIdx.x >> 1), n_tiles - 1);
+  const bool pad_pair = (int)(blockIdx.x >> 1) >= n_tiles;   // a pair past the last tile would redo it, unseen
   const int m0 = tile * TM;                    // the pair's 128-row tile
-  constexpr uint16_t ALL_MASK = (uint16_t)((1u << CS) - 1);
   const uint16_t pair_mask = (uint16_t)(3u << lead);
 
   if (tid == 0) {
-    // "full": TMAP -> only the leader's barrier is used: one expect_tx arrival covering both CTAs' bytes;
-    //         else the leader's collects its own TMA (expect_tx arrival) and the peer's relay arrival.
-    for (int i = 0; i < P_NST; ++i) { mbar_init(&bar_full[i], (rank == 0 && !TMAP) ? 2 : 1); mbar_init(&bar_empty[i], CS / 2); }
-    // hand-over barriers: RELAY -> 8 local warps (+ 1 relay arrival on the leader); else 8 warps x 2 CTAs on the leader
-    const int nh = RELAY ? (rank == 0 ? 9 : 8) : 16;
-    for (int i = 0; i < 4; ++i) { mbar_init(&bar_h[i], nh); mbar_init(&bar_rh[i], nh); }
+    // "full": the leader's collects its own TMA (expect_tx arrival) and the peer's relay arrival
+    for (int i = 0; i < P_NST; ++i) { mbar_init(&bar_full[i], rank == 0 ? 2 : 1); mbar_init(&bar_empty[i], 1); }
+    // hand-over barriers: 8 warps x 2 CTAs on the leader
+    for (int i = 0; i < 4; ++i) { mbar_init(&bar_h[i], 16); mbar_init(&bar_rh[i], 16); }
     mbar_init(&bar_r, 1); mbar_init(&bar_u, 1); mbar_init(&bar_c, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -244,39 +231,20 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_augru_pair2(const __grid_consta
       // ===== TMA producer: this CTA's half of the 24-stage weight stream of a step, 64 times =====
       if (lane == 0) {
         int stage = 0; uint32_t phase = 0;
-        if (TMAP) {
-          const CUtensorMap* tm = &pp.tmap[blockIdx.y];
-          const uint32_t full0_leader = mapa_rank(smem_u32(&bar_full[0]), lead);
-          const uint32_t sB_u = smem_u32(sB);
-          // CS > 2: the two CTAs of pair 0 each multicast THEIR column half to the same-parity CTA of every pair
-          uint16_t mc_mask = 0;
-          for (int c = (int)rank; c < CS; c += 2) mc_mask |= (uint16_t)(1u << c);
-          for (int t = 0; t < STEPS; ++t) {
-            int row = (int)rank * P_STAGES_PER_STEP * P2_TM_BOX_ROWS;
-            for (int i = 0; i < P_STAGES_PER_STEP; ++i, row += P2_TM_BOX_ROWS) {
-              mbar_wait(&bar_empty[stage], phase ^ 1);          // every pair of the cluster has released the stage
-              if (rank == 0) mbar_expect_tx(&bar_full[stage], 2 * P_STAGE_BYTES);
-              if (CS == 2) tma_box_cg2(sB_u + stage * P_STAGE_BYTES, tm, 0, row, full0_leader + stage * 8);
-              else if (crank < 2) tma_box_cg2_mc(sB_u + stage * P_STAGE_BYTES, tm, 0, row, full0_leader + stage * 8, mc_mask);
-              if (++stage == P_NST) { stage = 0; phase ^= 1; }
-            }
-          }
-        } else {
-          const uint8_t* img = S.Wimg + (size_t)rank * P_RANK_IMAGE_BYTES;
-          for (int t = 0; t < STEPS; ++t) {
-            const uint8_t* src = img;
-            for (int i = 0; i < P_STAGES_PER_STEP; ++i, src += P_STAGE_BYTES) {
-              mbar_wait(&bar_empty[stage], phase ^ 1);
-              mbar_expect_tx(&bar_full[stage], P_STAGE_BYTES);
-              bulk_g2s(sB + stage * P_STAGE_BYTES, src, P_STAGE_BYTES, &bar_full[stage]);
-              if (++stage == P_NST) { stage = 0; phase ^= 1; }
-            }
+        const uint8_t* img = S.Wimg + (size_t)rank * P_RANK_IMAGE_BYTES;
+        for (int t = 0; t < STEPS; ++t) {
+          const uint8_t* src = img;
+          for (int i = 0; i < P_STAGES_PER_STEP; ++i, src += P_STAGE_BYTES) {
+            mbar_wait(&bar_empty[stage], phase ^ 1);
+            mbar_expect_tx(&bar_full[stage], P_STAGE_BYTES);
+            bulk_g2s(sB + stage * P_STAGE_BYTES, src, P_STAGE_BYTES, &bar_full[stage]);
+            if (++stage == P_NST) { stage = 0; phase ^= 1; }
           }
         }
       }
     } else if (warp == 8 && rank == 1) {
-      // ===== ring relay (only without the tensor map): tell the leader that this CTA's copy of stage s has landed =====
-      if (!TMAP && lane == 0) {
+      // ===== ring relay: tell the leader that this CTA's copy of stage s has landed =====
+      if (lane == 0) {
         const uint32_t remote0 = mapa_rank(smem_u32(&bar_full[0]), lead);
         int stage = 0; uint32_t phase = 0;
         for (int i = 0; i < STEPS * P_STAGES_PER_STEP; ++i) {
@@ -300,27 +268,16 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_augru_pair2(const __grid_consta
         long long wacc[2] = {0, 0};
         long long* wa = dbg ? wacc : nullptr;
         if (dbg) dbg[1] = clock64();
-        issue_gate2<0>(leader, tbase, hHi_d, hLo_d, b_d, bar_full, bar_empty, bar_h, par, ALL_MASK, wa);   // chases phase C of step t-1
+        issue_gate2<0>(leader, tbase, hHi_d, hLo_d, b_d, bar_full, bar_empty, bar_h, par, wa);   // chases phase C of step t-1
         if (leader) commit2_mask(&bar_r, pair_mask);
         if (dbg) dbg[2] = clock64();
-        issue_gate2<1>(leader, tbase, hHi_d, hLo_d, b_d, bar_full, bar_empty, nullptr, 0, ALL_MASK, wa);
+        issue_gate2<1>(leader, tbase, hHi_d, hLo_d, b_d, bar_full, bar_empty, nullptr, 0, wa);
         if (leader) commit2_mask(&bar_u, pair_mask);
         if (dbg) dbg[3] = clock64();
         if (dbg) dbg[4] = clock64();
-        issue_gate2<2>(leader, tbase, rHi_d, rLo_d, b_d, bar_full, bar_empty, bar_rh, par, ALL_MASK, wa);  // chases phase R of this step
+        issue_gate2<2>(leader, tbase, rHi_d, rLo_d, b_d, bar_full, bar_empty, bar_rh, par, wa);  // chases phase R of this step
         if (leader) commit2_mask(&bar_c, pair_mask);
         if (dbg) { dbg[5] = clock64(); dbg[6] = wacc[0]; dbg[7] = wacc[1]; }
-      }
-    } else if (RELAY && rank == 1 && lane == 0) {
-      // ===== hand-over relays (peer CTA): forward each completed local phase with a cluster-scope release =====
-      // A barrier cannot complete its next phase before this one has been forwarded: that needs the leader's next gate on
-      // the same operand, which waits for this very arrival.  warp 11: the quarters of h; warp 10: the quarters of r*h.
-      if (warp == 11) {
-        for (int k = 0; k <= STEPS; ++k)
-          for (int i = 0; i < 4; ++i) { mbar_wait(&bar_h[i], k & 1); arrive_cl(bar_h_leader + i * 8); }
-      } else {
-        for (int t = 0; t < STEPS; ++t)
-          for (int i = 0; i < 4; ++i) { mbar_wait(&bar_rh[i], t & 1); arrive_cl(bar_rh_leader + i * 8); }
       }
     }
   } else {
@@ -343,13 +300,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_augru_pair2(const __grid_consta
     const float* st = S.scoresT + ((size_t)(m0 / TM) * STEPS) * TM + prow;
     const uint32_t tlane = tbase + ((uint32_t)(q * 32) << 16);
     const uint32_t a_row_off = (uint32_t)(rl / 8) * A_SBO + (uint32_t)(rl % 8) * 16 + (uint32_t)(hcb / 8) * LBO;
-    const bool local_arrive = RELAY || rank == 0;          // arrive on this CTA's own barrier (else: relaxed, on the leader's)
-    // publish quarter `i` of an A operand: this thread's stores -> async proxy, then one arrival per warp
+    // publish quarter `i` of an A operand: this thread's stores -> async proxy, then one arrival per warp on the leader's
+    // barrier
     auto publish = [&](uint64_t* bars, uint32_t bars_leader, int i) {
       tc_fence_before();
       proxy_fence();
       __syncwarp();
-      if (lane == 0) { if (local_arrive) mbar_arrive(&bars[i]); else arrive_remote(bars_leader + i * 8); }
+      if (lane == 0) { if (rank == 0) mbar_arrive(&bars[i]); else arrive_remote(bars_leader + i * 8); }
     };
     float h[64], x[4][16];
 #pragma unroll
@@ -365,14 +322,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_augru_pair2(const __grid_consta
     }
 #pragma unroll
     for (int i = 0; i < 4; ++i) publish(bar_h, bar_h_leader, i);
-#if R4_ABL & 4
-#define R4P2_LOADX(dst, base, colbase) do { _Pragma("unroll") for (int q_ = 0; q_ < 16; ++q_) (dst)[q_] = 0.125f * (float)(ln4 & 3); } while (0)
-#else
-#define R4P2_LOADX(dst, base, colbase) load_x16(dst, (base), (colbase), ln4)
-#endif
     // rolling input buffer: x[ch] always holds chunk ch of the NEXT phase to run (here: the r gate of step 0)
 #pragma unroll
-    for (int c4 = 0; c4 < 4; ++c4) { R4P2_LOADX(x[c4], xt, hcb + c4 * 32); }
+    for (int c4 = 0; c4 < 4; ++c4) load_x16(x[c4], xt, hcb + c4 * 32, ln4);
     float one_minus_s = 1.0f - __ldg(st);
 
     for (int t = 0; t < STEPS; ++t) {
@@ -399,16 +351,16 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_augru_pair2(const __grid_consta
         mbar_wait(&bar_r, par);
         if (dbg) dbg[9] = clock64();
         tc_fence_after();
-        P2_TMEM_LD16(tlane + P_TC_R + tcb, a[0]);
+        tmem_ld16(tlane + P_TC_R + tcb, a[0]);
 #pragma unroll
         for (int ch = 0; ch < 4; ++ch) {
           const int cur = ch & 1, nxt = cur ^ 1;
-          P2_TMEM_WAIT_LD();
-          if (ch < 3) P2_TMEM_LD16(tlane + P_TC_R + tcb + (ch + 1) * 32, a[nxt]);
+          tmem_wait_ld();
+          if (ch < 3) tmem_ld16(tlane + P_TC_R + tcb + (ch + 1) * 32, a[nxt]);
 #pragma unroll
           for (int j = 0; j < 16; ++j)
-            a[cur][j] = p2_rcp(1.0f + p2_ex2(fminf(preact2(a[cur][j], x[ch][j], P2_NL2E), 60.0f)), j) * h[ch * 16 + j];
-          R4P2_LOADX(x[ch], xs, HID + hcb + ch * 32);
+            a[cur][j] = rcp_approx(1.0f + ex2_approx(fminf(P2_NL2E * (a[cur][j] + x[ch][j]), 60.0f))) * h[ch * 16 + j];
+          load_x16(x[ch], xs, HID + hcb + ch * 32, ln4);
 #pragma unroll
           for (int g = 0; g < 2; ++g)
             split_store8(a[cur] + g * 8, sRhi, sRlo, a_row_off + (uint32_t)(ch * 4 + g) * LBO);
@@ -422,19 +374,19 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_augru_pair2(const __grid_consta
         mbar_wait(&bar_u, par);
         if (dbg) dbg[11] = clock64();
         tc_fence_after();
-        P2_TMEM_LD16(tlane + P_TC_U + tcb, a[0]);
+        tmem_ld16(tlane + P_TC_U + tcb, a[0]);
 #pragma unroll
         for (int ch = 0; ch < 4; ++ch) {
           const int cur = ch & 1, nxt = cur ^ 1;
-          P2_TMEM_WAIT_LD();
-          if (ch < 3) P2_TMEM_LD16(tlane + P_TC_U + tcb + (ch + 1) * 32, a[nxt]);
+          tmem_wait_ld();
+          if (ch < 3) tmem_ld16(tlane + P_TC_U + tcb + (ch + 1) * 32, a[nxt]);
 #pragma unroll
           for (int j = 0; j < 16; ++j)
-            a[cur][j] = 1.0f + p2_ex2(fminf(preact2(a[cur][j], x[ch][j], P2_NL2E), 60.0f));
-          R4P2_LOADX(x[ch], xs, 2 * HID + hcb + ch * 32);
-          P2_TMEM_ST16(tlane + P_TC_U + tcb + ch * 32, a[cur]);
+            a[cur][j] = 1.0f + ex2_approx(fminf(P2_NL2E * (a[cur][j] + x[ch][j]), 60.0f));
+          load_x16(x[ch], xs, 2 * HID + hcb + ch * 32, ln4);
+          tmem_st16(tlane + P_TC_U + tcb + ch * 32, a[cur]);
         }
-        P2_TMEM_WAIT_ST();
+        tmem_wait_st();
       }
       if (dbg) dbg[12] = clock64();
       // ---- phase C (the next step's r MMAs chase it quarter by quarter): c = tanh(acc_c + Xc) = 1 - 2/(1 + F), u = 1/E
@@ -444,28 +396,28 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_augru_pair2(const __grid_consta
         mbar_wait(&bar_c, par);
         if (dbg) dbg[13] = clock64();
         tc_fence_after();
-        P2_TMEM_LD16(tlane + P_TC_C + tcb, a[0]);
-        P2_TMEM_LD16(tlane + P_TC_U + tcb, u[0]);
+        tmem_ld16(tlane + P_TC_C + tcb, a[0]);
+        tmem_ld16(tlane + P_TC_U + tcb, u[0]);
 #pragma unroll
         for (int ch = 0; ch < 4; ++ch) {
           const int cur = ch & 1, nxt = cur ^ 1;
-          P2_TMEM_WAIT_LD();
+          tmem_wait_ld();
           if (ch < 3) {
-            P2_TMEM_LD16(tlane + P_TC_C + tcb + (ch + 1) * 32, a[nxt]);
-            P2_TMEM_LD16(tlane + P_TC_U + tcb + (ch + 1) * 32, u[nxt]);
+            tmem_ld16(tlane + P_TC_C + tcb + (ch + 1) * 32, a[nxt]);
+            tmem_ld16(tlane + P_TC_U + tcb + (ch + 1) * 32, u[nxt]);
           }
 #pragma unroll
           for (int j = 0; j < 16; ++j) {
-            const float F = 1.0f + p2_ex2(fminf(preact2(a[cur][j], x[ch][j], P2_2L2E), 60.0f));
+            const float F = 1.0f + ex2_approx(fminf(P2_2L2E * (a[cur][j] + x[ch][j]), 60.0f));
             const float E = u[cur][j];
-            const float rc = p2_rcp(E * F, j);                      // E, F <= 1 + 2^60: the product is finite
+            const float rc = rcp_approx(E * F);                      // E, F <= 1 + 2^60: the product is finite
             const float c = fmaf(-2.0f, rc * E, 1.0f);               // tanh
             const float up = one_minus_s * (rc * F);                 // (1 - s) sigmoid
             const float hn = fmaf(up, h[ch * 16 + j] - c, c);        // u' h + (1 - u') c
             h[ch * 16 + j] = hn;
             a[cur][j] = hn;
           }
-          R4P2_LOADX(x[ch], xs_next, hcb + ch * 32);      // (last step: a harmless re-read of this step's lines)
+          load_x16(x[ch], xs_next, hcb + ch * 32, ln4);      // (last step: a harmless re-read of this step's lines)
 #pragma unroll
           for (int g = 0; g < 2; ++g)
             split_store8(a[cur] + g * 8, sHhi, sHlo, a_row_off + (uint32_t)(ch * 4 + g) * LBO);
@@ -475,7 +427,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_augru_pair2(const __grid_consta
       if (dbg) dbg[14] = clock64();
       one_minus_s = oms_next;
     }
-#undef R4P2_LOADX
     if (valid) {
       float* o = S.out + (size_t)(m0 + prow) * p.out_ld + hcb;
 #pragma unroll
@@ -489,31 +440,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_augru_pair2(const __grid_consta
   __syncthreads();
   cluster_sync_all();                         // neither CTA frees TMEM / exits while the pair's MMAs or arrivals are in flight
   if (warp == 8) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" :: "r"(tbase), "r"(512));
-}
-
-// host: the pair weight image of one sequence (2 ranks x 24 stages x 16 KB, device pointer) as a tensor map of
-// [768 rows][256 x u32]; box = 256 x 16 = one ring stage.  cuTensorMapEncodeTiled is fetched through the runtime
-// (cudaGetDriverEntryPoint), so the library does not link libcuda.  Returns 0 on success.
-inline int make_pair_tensor_map(const void* dev_img, CUtensorMap* out) {
-  typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                               const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                               CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  static EncodeFn fn = [] {
-    void* f = nullptr;
-    cudaDriverEntryPointQueryResult qr;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &qr) != cudaSuccess || qr != cudaDriverEntryPointSuccess)
-      f = nullptr;
-    return reinterpret_cast<EncodeFn>(f);
-  }();
-  if (!fn) return 1;
-  const cuuint64_t gdim[2] = {256, (cuuint64_t)(2 * P_RANK_IMAGE_BYTES / P2_TM_ROW_BYTES)};
-  const cuuint64_t gstride[1] = {P2_TM_ROW_BYTES};
-  const cuuint32_t box[2] = {256, (cuuint32_t)P2_TM_BOX_ROWS};
-  const cuuint32_t estr[2] = {1, 1};
-  CUresult rc = fn(out, CU_TENSOR_MAP_DATA_TYPE_UINT32, 2, const_cast<void*>(dev_img), gdim, gstride, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return rc == CUDA_SUCCESS ? 0 : 2;
 }
 
 }  // namespace r4tc

@@ -22,8 +22,11 @@
 //     the other recurrence fills the gap;
 //   * registers: a thread owns one row x 64 columns of BOTH states (128 registers); gate inputs are walked in 8-column
 //     chunks with a 3-deep rolling prefetch that runs across phase boundaries (32 registers), 16 + 16 for accumulators;
-//   * the weight ring carries 48 stages per step (8 revolutions of the 6 stages: stage and parity stay compile-time).
-// Same arithmetic, weight image, tensor-map ring and release-relay hand-over as k_augru_pair2 (r4_augru_pair2.cuh).
+//   * the weight ring carries 48 stages per step (16 revolutions of the 3 stages: stage and parity stay compile-time).
+// Same arithmetic, weight image and hand-over as k_augru_pair2 (r4_augru_pair2.cuh).  The weight ring is fed by
+// tensor-map TMA: both CTAs issue cp.async.bulk.tensor.2d.cta_group::2 for their own half of the stage with the LEADER's
+// "full" barrier as the completion target, and the leader's producer posts one expect_tx for both halves -- no relay
+// thread, no remote arrive: the transaction count is the signal.
 #pragma once
 #include "r4_augru_pair2.cuh"
 
@@ -34,6 +37,15 @@ constexpr int PP_SMEM_BYTES = 2 * PP_SLOT_BYTES + P_NST * P_STAGE_BYTES + 128;
 constexpr int PP_USES = 2 * P_STAGES_PER_STEP;                   // 48 ring uses per step
 static_assert(PP_USES % (2 * P_NST) == 0, "stage parity must repeat every step");
 constexpr int PP_CH = 8, PP_NCH = 64 / PP_CH, PP_XD = 3;        // chunk width, chunks per phase, prefetch distance
+constexpr int P2_TM_ROW_BYTES = 1024;                             // tensor-map row = 256 x u32
+constexpr int P2_TM_BOX_ROWS = P_STAGE_BYTES / P2_TM_ROW_BYTES;   // 16 rows per ring stage
+
+// this CTA's 16 KB box of the weight image -> own shared memory, completion bytes -> the barrier at `mbar_cluster`
+// (a shared::cluster address: the leader's "full" barrier for both CTAs of the pair)
+__device__ __forceinline__ void tma_box_cg2(uint32_t dst_smem, const CUtensorMap* tm, int c0, int c1, uint32_t mbar_cluster) {
+  asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
+               :: "r"(dst_smem), "l"(reinterpret_cast<uint64_t>(tm)), "r"(c0), "r"(c1), "r"(mbar_cluster) : "memory");
+}
 
 __device__ __forceinline__ void tmem_ld8(uint32_t taddr, float* v) {
   uint32_t* u = reinterpret_cast<uint32_t*>(v);
@@ -66,7 +78,7 @@ __device__ __forceinline__ void issue_gate_pp(uint32_t leader, uint32_t d_tmem, 
     const int u = U0 + s8;
     const int stage = u % P_NST;
     const uint32_t par = (uint32_t)((u / P_NST) & 1);
-    const int kb = pair_kb(s8);                     // the weight image's order (r4_augru_pair.cuh), every gate
+    const int kb = pair_kb(s8);                     // the weight image's order (build_pair_image), every gate
     if (half_bar != nullptr && s8 == NKB / 2) { mbar_wait_cl(half_bar, half_par); tc_fence_after(); }
     mbar_wait(&bar_full[stage], par);
     if (leader) {
@@ -94,7 +106,6 @@ struct PpLane {
   uint8_t *aHi, *aLo;   // A operand of this recurrence (this CTA)
 };
 
-template <int RELAY>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) k_augru_pp(const __grid_constant__ AugruPairParams pp) {
   extern __shared__ uint8_t smem_raw[];
   __shared__ uint64_t bar_full[P_NST], bar_empty[P_NST], bar_h[2], bar_rh[2], bar_u[2], bar_c[2];
@@ -108,9 +119,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) k_augru
 
   if (tid == 0) {
     for (int i = 0; i < P_NST; ++i) { mbar_init(&bar_full[i], 1); mbar_init(&bar_empty[i], 1); }
-    const int nh = RELAY ? (rank == 0 ? 9 : 8) : 16;
     for (int s = 0; s < 2; ++s) {
-      mbar_init(&bar_h[s], nh); mbar_init(&bar_rh[s], nh);
+      mbar_init(&bar_h[s], 16); mbar_init(&bar_rh[s], 16);
       mbar_init(&bar_u[s], 1); mbar_init(&bar_c[s], 1);
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -180,18 +190,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) k_augru
         if (leader) commit2(&bar_c[1]);
         if (dbg) dbg[8] = clock64();
       }
-    } else if (RELAY && rank == 1 && lane == 0) {
-      // ===== hand-over relays (peer CTA; see r4_augru_pair2.cuh): warp 10 -> r*h, warp 11 -> h, each in the fixed time
-      // order  recurrence 0, recurrence 1  =====
-      if (warp == 10) {
-        const uint32_t dst[2] = {mapa_rank(smem_u32(&bar_rh[0]), 0), mapa_rank(smem_u32(&bar_rh[1]), 0)};
-        for (int t = 0; t < STEPS; ++t)
-          for (int s = 0; s < 2; ++s) { mbar_wait(&bar_rh[s], t & 1); arrive_cl(dst[s]); }
-      } else if (warp == 11) {
-        const uint32_t dst[2] = {mapa_rank(smem_u32(&bar_h[0]), 0), mapa_rank(smem_u32(&bar_h[1]), 0)};
-        for (int k = 0; k <= STEPS; ++k)
-          for (int s = 0; s < 2; ++s) { mbar_wait(&bar_h[s], k & 1); arrive_cl(dst[s]); }
-      }
     }
   } else {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 232;");
@@ -206,7 +204,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) k_augru
     if (!valid) r = p.R - 1;
     const uint32_t tlane = tbase + ((uint32_t)(q * 32) << 16);
     const uint32_t a_row_off = (uint32_t)(rl / 8) * A_SBO + (uint32_t)(rl % 8) * 16;
-    const bool local_arrive = RELAY || rank == 0;
     PpLane L[2];
 #pragma unroll
     for (int s = 0; s < 2; ++s) {
@@ -222,7 +219,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) k_augru
 #pragma unroll
     for (int s = 0; s < 2; ++s) { h_leader[s] = mapa_rank(smem_u32(&bar_h[s]), 0); rh_leader[s] = mapa_rank(smem_u32(&bar_rh[s]), 0); }
     auto arrive = [&](uint64_t* local, uint32_t remote) {      // lane 0, after proxy_fence + __syncwarp
-      if (local_arrive) mbar_arrive(local); else arrive_remote(remote);
+      if (rank == 0) mbar_arrive(local); else arrive_remote(remote);
     };
     float h[2][64], x[PP_XD + 1][PP_CH];
 #pragma unroll
@@ -282,7 +279,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) k_augru
             if (ch + PP_XD < PP_NCH) load_x8(x[(ch + PP_XD) % (PP_XD + 1)], xs, hc0 + (ch + PP_XD) * PP_CH, L[s].ln4);
 #pragma unroll
             for (int j = 0; j < PP_CH; ++j)
-              a[cur][j] = rcp_sel(1.0f + ex2_approx(fminf(P2_NL2E * (a[cur][j] + x[ch % (PP_XD + 1)][j]), 60.0f)), j) * h[s][ch * PP_CH + j];
+              a[cur][j] = rcp_approx(1.0f + ex2_approx(fminf(P2_NL2E * (a[cur][j] + x[ch % (PP_XD + 1)][j]), 60.0f))) * h[s][ch * PP_CH + j];
             split_store8(a[cur], L[s].aHi, L[s].aLo, a_row_off + (uint32_t)((hc0 + ch * PP_CH) / 8) * LBO);
           }
         }
@@ -339,7 +336,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) k_augru
             for (int j = 0; j < PP_CH; ++j) {
               const float F = 1.0f + ex2_approx(fminf(P2_2L2E * (a[cur][j] + x[xi][j]), 60.0f));
               const float E = u[cur][j];
-              const float rc = rcp_sel(E * F, j);
+              const float rc = rcp_approx(E * F);
               const float c = fmaf(-2.0f, rc * E, 1.0f);
               const float up = oms[s] * (rc * F);
               const float hn = fmaf(up, h[s][ch * PP_CH + j] - c, c);
@@ -376,6 +373,31 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1) k_augru
   __syncthreads();
   cluster_sync_all();
   if (warp == 8) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" :: "r"(tbase), "r"(512));
+}
+
+// host: the pair weight image of one sequence (2 ranks x 24 stages x 16 KB, device pointer) as a tensor map of
+// [768 rows][256 x u32]; box = 256 x 16 = one ring stage.  cuTensorMapEncodeTiled is fetched through the runtime
+// (cudaGetDriverEntryPoint), so the library does not link libcuda.  Returns 0 on success.
+inline int make_pair_tensor_map(const void* dev_img, CUtensorMap* out) {
+  typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                               const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                               CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+  static EncodeFn fn = [] {
+    void* f = nullptr;
+    cudaDriverEntryPointQueryResult qr;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &qr) != cudaSuccess || qr != cudaDriverEntryPointSuccess)
+      f = nullptr;
+    return reinterpret_cast<EncodeFn>(f);
+  }();
+  if (!fn) return 1;
+  const cuuint64_t gdim[2] = {256, (cuuint64_t)(2 * P_RANK_IMAGE_BYTES / P2_TM_ROW_BYTES)};
+  const cuuint64_t gstride[1] = {P2_TM_ROW_BYTES};
+  const cuuint32_t box[2] = {256, (cuuint32_t)P2_TM_BOX_ROWS};
+  const cuuint32_t estr[2] = {1, 1};
+  CUresult rc = fn(out, CU_TENSOR_MAP_DATA_TYPE_UINT32, 2, const_cast<void*>(dev_img), gdim, gstride, box, estr,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  return rc == CUDA_SUCCESS ? 0 : 2;
 }
 
 }  // namespace r4tc

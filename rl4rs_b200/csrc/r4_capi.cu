@@ -2,9 +2,6 @@
 // kernels of r4_kernels.cuh.  No torch, no Python: plain CUDA runtime.  See DESIGN.md.
 #include "../../include/rl4rs_b200.h"
 #include "r4_kernels.cuh"
-#include "r4_augru_tc.cuh"
-#include "r4_augru_pair.cuh"
-#include "r4_augru_pair2.cuh"
 #include "r4_augru_pp.cuh"
 #include "r4_gemm_tc.cuh"
 #include "r4_scores_tc.cuh"
@@ -43,8 +40,8 @@ struct PerSeq {
   float *au_wx = nullptr, *au_bx = nullptr, *au_wgh = nullptr, *au_wch = nullptr;
   float *wqd = nullptr, *wp = nullptr, *ab1 = nullptr, *aw2 = nullptr, *ab2 = nullptr, *akv = nullptr;
   uint8_t *gru_wx_img = nullptr, *au_wx_img = nullptr, *wp_img = nullptr, *gru_img = nullptr;   // pre-tiled bf16 hi/lo images of the input projections
-  uint8_t* au_pair_img = nullptr;   // the same weights tiled per CTA rank for the 2-CTA kernel (r4_augru_pair.cuh)
-  CUtensorMap au_pair_tmap;    // au_pair_img as a 2-D tensor of 1 KB rows (r4_augru_pair2.cuh: tensor-map TMA ring)
+  uint8_t* au_pair_img = nullptr;   // the same weights tiled per CTA rank for the 2-CTA kernel (r4_augru_pair2.cuh)
+  CUtensorMap au_pair_tmap;    // au_pair_img as a 2-D tensor of 1 KB rows (r4_augru_pp.cuh: tensor-map TMA ring)
   bool au_pair_tmap_ok = false;
   float abk = 0.f;
 };
@@ -287,21 +284,15 @@ int build_cache(r4_env* e, int si, const int32_t* ids, int n, SeqCache& c, cudaS
 // Kernel-choice options (r4_set_option; the environment gives the initial values).
 struct AugruOpts {
   int force = 0;          // 0 rule, 2 pair kernel (one recurrence per pair), 3 ping-pong pair kernel (1 was the deleted one-CTA kernel)
-  int pair_impl = 1;      // k_augru_pair2<RELAY, TMAP>: 1 = <0,0> (default), 2 = <0,1>, 3 = <1,0>, 4 = <1,1>; k_augru_pp<RELAY> follows RELAY
   // cost of one wave, measured (tools/augru_probe.cu, round 2, ms x 25): k_augru_pair2 0.51 ms per 74 tile-sequences,
   // k_augru_pp 0.96 ms per 74 TILES (= 148 tile-sequences)
   int cost_pair = 13, cost_pp = 24;
-  int cluster = 2;        // CTAs per cluster of the pair kernel: 2, or 4 / 8 = weight stream shared by 2 / 4 pairs (multicast)
-  int scores_impl = 2;    // 2 = k_scores_tc2 (both attention layers on the tensor pipe), 1 = k_scores_tc (second layer as FFMA2)
   int scores_shared_pct = 85;    // k_scores_tc2: CTA share of a shared (L2-resident) sequence, per cent of an even split (tools/scores_probe.cu,
                                  // us per 4096-row pass: 100 % 98.5, 85 % 86.8, 75 % 90.1, 65 % 100.6, 55 % 120.8)
   int pay_obs_reuse = 1;  // a paying step takes its observation from its reward pass (r4_step); 0 = separate observation pass
   AugruOpts() {
     if (getenv("R4_NO_PAY_OBS_REUSE")) pay_obs_reuse = 0;
-    if (const char* e = getenv("R4_SCORES_IMPL")) { int v = atoi(e); if (v == 1 || v == 2) scores_impl = v; }
     if (getenv("R4_AUGRU_PAIR")) force = 2; else if (getenv("R4_AUGRU_PP")) force = 3;
-    if (const char* e = getenv("R4_AUGRU_PAIR_IMPL")) { int v = atoi(e); if (v >= 1 && v <= 4) pair_impl = v; }
-    if (const char* e = getenv("R4_AUGRU_CLUSTER")) { int v = atoi(e); if (v == 2 || v == 4 || v == 8) cluster = v; }
     if (const char* e = getenv("R4_AUGRU_RULE")) {
       int a = 0, b = 0;
       if (sscanf(e, "%d,%d", &a, &b) == 2 && a > 0 && b > 0) { cost_pair = a; cost_pp = b; }
@@ -325,7 +316,6 @@ static int augru_choice(int ctas) {
   const int force = augru_opts().force;
   return force ? force : augru_rule(ctas, sms);
 }
-static int augru_pair_impl() { return augru_opts().pair_impl; }
 
 // One simulator pass over `R` feature rows (cat/dense already assembled, chunk-local pointers).
 int forward_rows(r4_env* e, int R, int row0, int div, const int32_t* cat, const float* dense,
@@ -463,7 +453,6 @@ int forward_rows(r4_env* e, int R, int row0, int div, const int32_t* cat, const 
   // around a kernel on the low-priority side stream would time its wait for free SMs, not the kernel.
   static const bool no_side_env = getenv("R4_NO_SIDE_STREAM") != nullptr;
   const bool no_side = no_side_env || e->prof_mode == 2;
-  static const bool side_early = getenv("R4_SIDE_EARLY") != nullptr;    // diagnostics: fork before k_query (old schedule)
   auto side_work = [&]() -> int {
     cudaStream_t ss = no_side ? st : e->side;
     if (!no_side) R4_CUDA(e, cudaStreamWaitEvent(e->side, e->ev_fork, 0));
@@ -476,56 +465,35 @@ int forward_rows(r4_env* e, int R, int row0, int div, const int32_t* cat, const 
     if (!no_side) R4_CUDA(e, cudaEventRecord(e->ev_join, ss));
     return R4_OK;
   };
-  if (no_side || side_early) {
-    if (!no_side) R4_CUDA(e, cudaEventRecord(e->ev_fork, st));
-    if ((rc = side_work())) return rc;
-  }
+  if (no_side && (rc = side_work())) return rc;
   { ProfScope ps(e, SL_MISC, st, (double)R);
     r4tc::k_query<<<(R + 7) / 8, 128, 0, st>>>(R, cat, e->emb_seq, e->ps[0].wqd, e->ps[0].ab1, e->ps[1].wqd, e->ps[1].ab1,
                                                 qbuf, qa0, qa1); }
   R4_LAUNCH_CHECK(e, "k_query");
   { ProfScope ps(e, SL_SCORES, st, (double)R * 2 * MAXLEN * 2.0 * (EMB * AH1 + AH1 * AH2 + AH2));
     const int nt = (R + 1) / 2;
-    if (augru_opts().scores_impl == 1) r4tc::k_scores_tc<<<dim3(std::min(nt, 74), 2), r4tc::S_THREADS, r4tc::S_SMEM_BYTES, st>>>(sp, cat, e->emb_seq);
-    else {
-      const int ctas = std::min(2 * nt, 148);
-      r4tc::k_scores_tc2<false><<<ctas, r4tc::S2_THREADS, r4tc::S2_SMEM_BYTES, st>>>(
-          sp, r4tc::scores_grid_split(ctas, nt, sh[0], sh[1], augru_opts().scores_shared_pct));
-    } }
+    const int ctas = std::min(2 * nt, 148);
+    r4tc::k_scores_tc2<false><<<ctas, r4tc::S2_THREADS, r4tc::S2_SMEM_BYTES, st>>>(
+        sp, r4tc::scores_grid_split(ctas, nt, sh[0], sh[1], augru_opts().scores_shared_pct)); }
   R4_LAUNCH_CHECK(e, "k_scores_tc");
-  if (!no_side && !side_early) R4_CUDA(e, cudaEventRecord(e->ev_fork, st));
+  if (!no_side) R4_CUDA(e, cudaEventRecord(e->ev_fork, st));
   { ProfScope ps(e, SL_AUGRU, st, (double)R * 2 * MAXLEN * 2.0 * (AUH * 2 * AUH + AUH * AUH));
-    const dim3 pgrid(rtiles * 2, 2);
-    const int which = augru_choice(2 * rtiles);
-    if (which == 3) {
-      r4tc::AugruPairParams pp;
-      pp.b = rp; pp.tmap[0] = e->ps[0].au_pair_tmap; pp.tmap[1] = e->ps[1].au_pair_tmap;
-      if (augru_pair_impl() >= 3) r4tc::k_augru_pp<1><<<dim3(rtiles * 2), r4tc::NTHREADS, r4tc::PP_SMEM_BYTES, st>>>(pp);
-      else r4tc::k_augru_pp<0><<<dim3(rtiles * 2), r4tc::NTHREADS, r4tc::PP_SMEM_BYTES, st>>>(pp);
+    r4tc::AugruPairParams pp;
+    pp.b = rp; pp.tmap[0] = e->ps[0].au_pair_tmap; pp.tmap[1] = e->ps[1].au_pair_tmap;
+    if (augru_choice(2 * rtiles) == 3) {
+      r4tc::k_augru_pp<<<dim3(rtiles * 2), r4tc::NTHREADS, r4tc::PP_SMEM_BYTES, st>>>(pp);
     } else {
-      r4tc::AugruPairParams pp;
-      pp.b = rp; pp.tmap[0] = e->ps[0].au_pair_tmap; pp.tmap[1] = e->ps[1].au_pair_tmap;
-      // cluster size = CTAs sharing one weight stream (2 = one pair, 4 / 8 = 2 / 4 pairs: multicast ring)
-      const int cs = augru_opts().cluster;
+      // one 2-CTA cluster per tile and sequence
       cudaLaunchConfig_t lc = {};
       cudaLaunchAttribute at[1];
       at[0].id = cudaLaunchAttributeClusterDimension;
-      at[0].val.clusterDim.x = cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-      lc.gridDim = dim3((pgrid.x + cs - 1) / cs * cs, 2); lc.blockDim = dim3(r4tc::NTHREADS);
+      at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+      lc.gridDim = dim3(rtiles * 2, 2); lc.blockDim = dim3(r4tc::NTHREADS);
       lc.dynamicSmemBytes = r4tc::P_SMEM_BYTES; lc.stream = st; lc.attrs = at; lc.numAttrs = 1;
-      cudaError_t le;
-      if (cs == 4) le = cudaLaunchKernelEx(&lc, r4tc::k_augru_pair2<0, 1, 4>, pp);
-      else if (cs == 8) le = cudaLaunchKernelEx(&lc, r4tc::k_augru_pair2<0, 1, 8>, pp);
-      else switch (augru_pair_impl()) {
-        case 2: le = cudaLaunchKernelEx(&lc, r4tc::k_augru_pair2<0, 1, 2>, pp); break;
-        case 3: le = cudaLaunchKernelEx(&lc, r4tc::k_augru_pair2<1, 0, 2>, pp); break;
-        case 4: le = cudaLaunchKernelEx(&lc, r4tc::k_augru_pair2<1, 1, 2>, pp); break;
-        default: le = cudaLaunchKernelEx(&lc, r4tc::k_augru_pair2<0, 0, 2>, pp); break;
-      }
-      (void)le;
+      (void)cudaLaunchKernelEx(&lc, r4tc::k_augru_pair2, pp);
     } }
   R4_LAUNCH_CHECK(e, augru_choice(2 * rtiles) == 3 ? "k_augru_pp" : "k_augru_pair2");
-  if (!no_side && !side_early && (rc = side_work())) return rc;
+  if (!no_side && (rc = side_work())) return rc;
   if (!no_side) R4_CUDA(e, cudaStreamWaitEvent(st, e->ev_join, 0));
   float* obs = obs_out;
   if (!obs) {
@@ -697,16 +665,9 @@ int r4_create(const r4_config* cfg, int device, r4_env** out) {
             cudaMalloc(&e->sflag, (size_t)e->B) == cudaSuccess;
   if (!ok) { r4_destroy(e); return fail(nullptr, R4_ERR_NOMEM, "r4_create: cudaMalloc failed"); }
   cudaFuncSetAttribute(r4tc::k_gru_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::G1_SMEM_BYTES);
-  cudaFuncSetAttribute(r4tc::k_augru_pair2<0, 1, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::P_SMEM_BYTES);
-  cudaFuncSetAttribute(r4tc::k_augru_pair2<0, 1, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::P_SMEM_BYTES);
-  cudaFuncSetAttribute(r4tc::k_augru_pp<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::PP_SMEM_BYTES);
-  cudaFuncSetAttribute(r4tc::k_augru_pp<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::PP_SMEM_BYTES);
-  cudaFuncSetAttribute(r4tc::k_augru_pair2<1, 1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::P_SMEM_BYTES);
-  cudaFuncSetAttribute(r4tc::k_augru_pair2<0, 1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::P_SMEM_BYTES);
-  cudaFuncSetAttribute(r4tc::k_augru_pair2<1, 0, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::P_SMEM_BYTES);
-  cudaFuncSetAttribute(r4tc::k_augru_pair2<0, 0, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::P_SMEM_BYTES);
+  cudaFuncSetAttribute(r4tc::k_augru_pp, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::PP_SMEM_BYTES);
+  cudaFuncSetAttribute(r4tc::k_augru_pair2, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::P_SMEM_BYTES);
   cudaFuncSetAttribute(r4tc::k_gemm_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::G_SMEM_BYTES);
-  cudaFuncSetAttribute(r4tc::k_scores_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::S_SMEM_BYTES);
   cudaFuncSetAttribute(r4tc::k_scores_tc2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, r4tc::S2_SMEM_BYTES);
   cudaFuncSetAttribute(k_cat_attn, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_CAT);
   cudaFuncSetAttribute(k_cat_pool, cudaFuncAttributeMaxDynamicSharedMemorySize, POOL_SMEM);
@@ -1149,12 +1110,9 @@ int r4_set_option(const char* key, int value) {
   AugruOpts& o = augru_opts();
   const std::string k(key);
   if (k == "augru_kernel" && (value == 0 || value == 2 || value == 3)) o.force = value;
-  else if (k == "augru_pair_impl" && value >= 1 && value <= 4) o.pair_impl = value;
   else if (k == "augru_cost_pair" && value > 0) o.cost_pair = value;
   else if (k == "augru_cost_pp" && value > 0) o.cost_pp = value;
-  else if (k == "augru_cluster" && (value == 2 || value == 4 || value == 8)) o.cluster = value;
   else if (k == "pay_obs_reuse" && (value == 0 || value == 1)) o.pay_obs_reuse = value;
-  else if (k == "scores_impl" && (value == 1 || value == 2)) o.scores_impl = value;
   else if (k == "scores_shared_pct" && value >= 10 && value <= 100) o.scores_shared_pct = value;
   else return fail(nullptr, R4_ERR_ARG, "r4_set_option: unknown key or value out of range: " + k);
   return R4_OK;

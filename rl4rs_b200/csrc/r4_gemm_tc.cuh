@@ -12,7 +12,7 @@
 // for W, 12-15 epilogue (TMEM -> bias/act -> global) on the second of two TMEM accumulators, 10-11 idle.
 // Operand ring: 2 stages x (A hi/mid/lo 24 KB + W hi/mid/lo <=48 KB), K block = 32; raw A ring: 4 x 16 KB.
 #pragma once
-#include "r4_augru_tc.cuh"
+#include "r4_tc_common.cuh"
 
 namespace r4tc {
 

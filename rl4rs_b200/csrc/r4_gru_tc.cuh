@@ -3,13 +3,13 @@
 //
 //   r = sigmoid(Xr_t + h Wr)   u = sigmoid(Xu_t + h Wu)   c = tanh(Xc_t + (r*h) Wc)   h <- u h + (1-u) c
 //
-// Same machinery as r4_augru_tc.cuh (bf16 hi/lo split x3 products, fp32 accumulators in TMEM, fp32 state in
+// Same machinery as the AUGRU kernels (bf16 hi/lo split x3 products, fp32 accumulators in TMEM, fp32 state in
 // registers, cp.async.bulk weight ring) but with hidden 128 everything fits without aliasing:
 //   TMEM  r | u | c = 3 x 128 columns;  shared: h operand 64 KB + SEPARATE r*h operand 64 KB + 4 x 8 KB ring,
 // so the u-GEMM runs while the epilogue converts r*h, and sigmoid(u) is written back in place during the c-GEMM.
 // One CTA = 128 sequences.  Warp roles: 8 epilogue warps (thread = row x 64-column half), MMA issuer, TMA producer.
 #pragma once
-#include "r4_augru_tc.cuh"
+#include "r4_tc_common.cuh"
 
 namespace r4tc {
 

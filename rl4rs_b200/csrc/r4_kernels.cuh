@@ -1,6 +1,6 @@
 // r4_kernels.cuh -- sm_100a kernels of the RL4RS hot path (SURVEY.md section 2a): the integer / gather half
 // (K1-K5, K10 tail, K11).  The GEMM-shaped half lives in r4_gemm_tc.cuh, r4_gru_tc.cuh, r4_scores_tc.cuh,
-// r4_augru_tc.cuh (tcgen05) and the policy/learner in r4_ppo.cuh.
+// r4_augru_pair2.cuh, r4_augru_pp.cuh (tcgen05) and the policy/learner in r4_ppo.cuh.
 //
 // Every kernel cites the reference operation it replaces.  Arithmetic is fp32 with precise
 // expf/tanhf/expm1f (parity: 1e-4 relative against the f32 CPU oracle); reward and kNN scores are

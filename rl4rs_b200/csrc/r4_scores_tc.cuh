@@ -5,23 +5,19 @@
 //   z1_t   = sigmoid(q (Wq+Wd) + b1 + k_t (Wk-Wd) + (q * k_t) Wp)       k_t = GRU-1 output t (cached H)
 //   z2_t   = sigmoid(z1_t W2 + b2);   score_t = z2_t . kv + b           (raw, unbounded)
 //
-// The only GEMM-shaped term, (q*k_t) Wp, is a [64 keys x 128] x [128 x 64] product per (row, sequence).  Two
-// feature rows are stacked into one UMMA tile (M = 128 key rows, N = 64, K = 128).  Persistent CTAs loop over
-// tiles; producer warps gather the 10 slate embeddings, build A = q*H as bf16 hi/lo core matrices (double
-// buffered), one lane issues 5 MMAs per K16 (A hi/lo x Wp hi/mid/lo: 2-way x 3-way split), epilogue warps
-// (lane = key) add q(Wq+Wd)+b1 and the cached key half, run the 64->16->1 tail in registers and write the
-// scores in the lane-major tile layout the AUGRU kernels read.
+// k_query computes q and the query half q (Wq+Wd) + b1 per feature row; k_scores_tc2 does the rest, both attention
+// layers on the tensor pipe, and writes the scores in the lane-major tile layout the AUGRU kernels read.
 #pragma once
-#include "r4_augru_tc.cuh"
+#include "r4_tc_common.cuh"
 #include "r4_gemm_tc.cuh"
 
 namespace r4tc {
 
 constexpr int S_K = 128, S_N = 64, S_KEYS = 64, AH2_N = 16;
-// A operand (built by the producer warps): K-adjacent core matrices 160 B apart instead of 128.  A producer quarter-warp
-// holds (2 rows x 4 K chunks) -- the mapping that keeps its global loads in whole 128-byte lines -- and with LBO = 128 the
-// four K chunks of a row hit the same banks: every 128-bit operand store replayed 4x and the kernel ran at 84 % of the
-// L1/shared pipe on those replays (ncu, round 2).  With 160 the bank group of (row, kc) is (row + 2 kc) mod 8: distinct.
+// A operand (built by the producer warps): K-adjacent core matrices 160 B apart instead of 128.  With LBO = 128 the K
+// chunks of a row hit the same banks: a producer quarter-warp that stored (2 rows x 4 K chunks) replayed every 128-bit
+// operand store 4x and ran the kernel at 84 % of the L1/shared pipe on those replays (ncu, round 2).  With 160 the bank
+// group of (row, kc) is (row + 2 kc) mod 8: distinct.
 constexpr int S_A_LBO = 160;
 constexpr int S_A_SBO = (S_K / 8) * S_A_LBO;       // 2560: 8-row groups of the A operand
 constexpr int S_A_SPLIT = (TM / 8) * S_A_SBO;      // 40 KB per split
@@ -29,11 +25,6 @@ constexpr int S_A_STAGE = 2 * S_A_SPLIT;           // hi + lo = 80 KB
 constexpr int S_B_SPLIT = S_N * S_K * 2;           // 16 KB per split
 constexpr int S_B_BYTES = 3 * S_B_SPLIT;           // 48 KB, resident
 constexpr int S_SBO = (S_K / 8) * 128;             // 2048: 8-row groups (B: the weight image)
-constexpr int S_SMEM_BYTES = 2 * S_A_STAGE + S_B_BYTES + 1024;
-constexpr int S_PROD_WARPS = 8, S_EPI_WARPS = 8;  // ncu, round 2: with 4 + 4 every SM sub-partition had ONE producer and ONE epilogue
-constexpr int S_W_MMA = S_PROD_WARPS + S_EPI_WARPS, S_W_LOAD = S_W_MMA + 1;   // warp, each a serial dependency chain: 20 k cycles per tile
-constexpr int S_THREADS = (S_W_LOAD + 1) * 32;     // 576: 8 producer + 8 epilogue + MMA + loader warps
-constexpr int S_TC_PART = 2 * S_N;                 // TMEM columns of the epilogue pairs' partial sums (2 buffers x 16)
 // cached key half k_t (Wk - Wd): Kp [n_cached][16 column quads][64 keys][4] (r4_gemm_tc.cuh: kq_index)
 
 // host: Wp [128 k][64 n] fp32 -> 3 splits of [64 n x 128 k] K-major core matrices
@@ -72,7 +63,7 @@ struct ScoreTcParams {
 };
 
 // q = reduce_mean(E_s[cat[-10:]]) and qa_i = q (Wq_i + Wd_i) + b1_i for both sequences (nets/utils.py:114-115 and
-// the query half of :121-122).  8 rows per CTA, 128 threads.  Keeping this out of k_scores_tc takes two dependent
+// the query half of :121-122).  8 rows per CTA, 128 threads.  Keeping this out of k_scores_tc2 takes two dependent
 // HBM round trips (category ids -> embedding rows) and a 128-long serial FMA chain off its per-tile critical path.
 __global__ void __launch_bounds__(128) k_query(int R, const int32_t* __restrict__ cat, const float* __restrict__ emb_seq,
                                                const float* __restrict__ Wqd0, const float* __restrict__ b10,
@@ -99,7 +90,7 @@ __global__ void __launch_bounds__(128) k_query(int R, const int32_t* __restrict_
 #pragma unroll
   for (int i = 0; i < 8; ++i) acc[i] = b;
   // 16 weight loads in flight per thread (with 4 the 128-long loop was 32 exposed L2 round trips; the kernel sits between
-  // k_assemble and k_scores_tc on the critical path of every pass)
+  // k_assemble and k_scores_tc2 on the critical path of every pass)
   for (int k0 = 0; k0 < S_K; k0 += 16) {
     float w[16];
 #pragma unroll
@@ -112,12 +103,6 @@ __global__ void __launch_bounds__(128) k_query(int R, const int32_t* __restrict_
   float* o = sq ? qa1 : qa0;
 #pragma unroll
   for (int i = 0; i < 8; ++i) if (r0 + i < R) o[(size_t)(r0 + i) * S_N + j] = acc[i];
-}
-
-// acc <- a * b + acc on two fp32 lanes at once (PTX fma.rn.f32x2, sm_100+): each lane rounds like a scalar fma.rn.f32
-__device__ __forceinline__ void ffma2(float2& acc, float2 a, float2 b) {
-  uint64_t& c = reinterpret_cast<uint64_t&>(acc);
-  asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(c) : "l"(reinterpret_cast<uint64_t&>(a)), "l"(reinterpret_cast<uint64_t&>(b)));
 }
 
 // packed fp32 pairs (sm_100+): each lane rounds like the scalar instruction
@@ -145,225 +130,24 @@ __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" :: "r"(id), "r"(nthreads) : "memory");
 }
 
-__global__ void __launch_bounds__(S_THREADS, 1) k_scores_tc(ScoreTcParams p, const int32_t* __restrict__ cat,
-                                                            const float* __restrict__ emb_seq) {
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* sA = smem;                           // 2 stages x (hi, lo)
-  uint8_t* sB = smem + 2 * S_A_STAGE;           // Wp hi/mid/lo
-  __shared__ uint64_t bar_afull[2], bar_aempty[2], bar_tfull[2], bar_tempty[2], bar_w;
-  __shared__ uint32_t tmem_base_s;
-  __shared__ __align__(16) float W2_s[S_N * 16];
-  __shared__ float b2_s[16], kv_s[16];
-  __shared__ __align__(16) float qa_s[2][2 * S_N];      // q (Wq+Wd) + b1 of the tile's two feature rows, double buffered
-  __shared__ __align__(16) float q_s[2][2 * S_K];       // the two query rows themselves (producers), double buffered
-  const ScoreTcSeq& S = p.s[blockIdx.y];
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int ntiles = (p.R + 1) / 2;
-
-  if (tid == 0) {
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&bar_afull[i], S_PROD_WARPS * 32); mbar_init(&bar_aempty[i], 1);
-      mbar_init(&bar_tfull[i], 1); mbar_init(&bar_tempty[i], S_EPI_WARPS * 32);
-    }
-    mbar_init(&bar_w, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == S_W_MMA) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(&tmem_base_s)), "r"(256));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
-  for (int i = tid; i < S_N * 16; i += S_THREADS) W2_s[i] = __ldg(S.W2 + i);
-  if (tid < 16) { b2_s[tid] = __ldg(S.b2 + tid); kv_s[tid] = __ldg(S.kv + tid); }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tbase = tmem_base_s;
-
-  if (warp == S_W_LOAD) {
-    if (lane == 0) {                                   // Wp image: once per CTA
-      mbar_expect_tx(&bar_w, S_B_BYTES);
-      bulk_g2s(sB, S.WpImg, S_B_BYTES, &bar_w);
-    }
-  } else if (warp == S_W_MMA) {
-    if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc(TM, S_N);
-      mbar_wait(&bar_w, 0);
-      const uint32_t b0 = smem_u32(sB);
-      int it = 0;
-      for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++it) {
-        const int s = it & 1;
-        const uint32_t ph = (it >> 1) & 1;
-        mbar_wait(&bar_afull[s], ph);
-        mbar_wait(&bar_tempty[s], ph ^ 1);
-        tc_fence_after();
-        const uint32_t a0 = smem_u32(sA + s * S_A_STAGE);
-        const uint32_t d = tbase + s * S_N;
-#pragma unroll
-        for (int j = 0; j < S_K / 16; ++j) {
-          const uint32_t ko = j * 2 * LBO, ka = j * 2 * S_A_LBO;
-          uint64_t ah = make_desc(a0 + ka, S_A_LBO, S_A_SBO), al = make_desc(a0 + S_A_SPLIT + ka, S_A_LBO, S_A_SBO);
-          uint64_t bh = make_desc(b0 + ko, LBO, S_SBO), bm = make_desc(b0 + S_B_SPLIT + ko, LBO, S_SBO);
-          uint64_t bl = make_desc(b0 + 2 * S_B_SPLIT + ko, LBO, S_SBO);
-          mma_bf16(d, al, bm, idesc, j ? 1u : 0u);
-          mma_bf16(d, ah, bl, idesc, 1u);
-          mma_bf16(d, al, bh, idesc, 1u);
-          mma_bf16(d, ah, bm, idesc, 1u);
-          mma_bf16(d, ah, bh, idesc, 1u);
-        }
-        umma_commit(&bar_aempty[s]);
-        umma_commit(&bar_tfull[s]);
-      }
-    }
-  } else if (warp < S_PROD_WARPS) {
-    // ===== producers: A = q * H as bf16 hi/lo; thread = (row slot tid / 4 of 64, K chunk tid % 4), 2 row passes =====
-    // All 16 H loads of a thread and tile (4 K blocks x 2 row passes x 32 B) are issued before the first one is used, and
-    // q comes from shared memory: ncu (round 2, second capture) had the producers waiting on two dependent HBM round trips
-    // per tile (the cached H of a 4096-row pass is 134 MB, it streams from HBM) with the epilogue warps waiting for them.
-    const int kc = tid & 3;
-    int it = 0;
-    for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++it) {
-      const int s = it & 1;
-      const uint32_t ph = (it >> 1) & 1;
-      if (tid < 64) {                              // the tile's two query rows: 2 x 128 floats
-        const int r = min(tile * 2 + (tid >> 5), p.R - 1);
-        reinterpret_cast<float4*>(q_s[s])[tid] = __ldg(reinterpret_cast<const float4*>(p.q + (size_t)r * S_K) + (tid & 31));
-      }
-      float4 hv[S_K / 32][2][2];
-#pragma unroll
-      for (int kb = 0; kb < S_K / 32; ++kb) {
-#pragma unroll
-        for (int i2 = 0; i2 < 2; ++i2) {
-          const int m = i2 * 64 + (tid >> 2);          // tile row: feature row m/64, key m%64
-          const int r = min(tile * 2 + (m >> 6), p.R - 1);
-          const size_t ci = S.shared ? 0 : (size_t)((p.row0 + r) / p.div);
-          const float* hp = S.H + (ci * S_KEYS + (m & 63)) * S_K + kb * 32 + kc * 8;
-          hv[kb][i2][0] = __ldg(reinterpret_cast<const float4*>(hp));
-          hv[kb][i2][1] = __ldg(reinterpret_cast<const float4*>(hp + 4));
-        }
-      }
-      named_bar_sync(3, S_PROD_WARPS * 32);        // q_s[s] is complete; it is rewritten two tiles later
-      mbar_wait(&bar_aempty[s], ph ^ 1);          // MMA finished reading this A stage
-      uint8_t* a = sA + s * S_A_STAGE;
-#pragma unroll
-      for (int kb = 0; kb < S_K / 32; ++kb) {
-#pragma unroll
-        for (int i2 = 0; i2 < 2; ++i2) {
-          const int m = i2 * 64 + (tid >> 2);
-          const int k = kb * 32 + kc * 8;
-          const float4 q0 = *reinterpret_cast<const float4*>(q_s[s] + (m >> 6) * S_K + k);
-          const float4 q1 = *reinterpret_cast<const float4*>(q_s[s] + (m >> 6) * S_K + k + 4);
-          const float4 h0 = hv[kb][i2][0], h1 = hv[kb][i2][1];
-          float v[8] = {h0.x * q0.x, h0.y * q0.y, h0.z * q0.z, h0.w * q0.w,
-                        h1.x * q1.x, h1.y * q1.y, h1.z * q1.z, h1.w * q1.w};
-          uint4 hi, lo;
-          split8(v, hi, lo);
-          const uint32_t off = (uint32_t)(m / 8) * S_A_SBO + (uint32_t)(k / 8) * S_A_LBO + (uint32_t)(m % 8) * 16;
-          *reinterpret_cast<uint4*>(a + off) = hi;
-          *reinterpret_cast<uint4*>(a + S_A_SPLIT + off) = lo;
-        }
-      }
-      proxy_fence();
-      mbar_arrive(&bar_afull[s]);
-    }
-  } else if (warp < S_W_MMA) {
-    // ===== epilogue: lane = key row of the tile; the two warps of a TMEM lane quarter split the 64 hidden units of the
-    // first attention layer (jh = 0: units 0-31, jh = 1: 32-63); jh = 1 hands its 16 partial sums of the second layer to
-    // its partner through 16 spare TMEM columns of their common lanes =====
-    const int e = (tid - S_PROD_WARPS * 32) & 127;   // row of the tile: 0..127
-    const int jh = (tid - S_PROD_WARPS * 32) >> 7;
-    const int ew = e >> 5;                       // TMEM lane quarter
-    const int rr = e >> 6, key = e & 63;
-    const int j0 = jh * (S_N / 2);
-    int it = 0;
-    for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++it) {
-      const int s = it & 1;
-      const uint32_t ph = (it >> 1) & 1;
-      const int r = tile * 2 + rr;
-      const int rc = min(r, p.R - 1);
-      const size_t ci = S.shared ? 0 : (size_t)((p.row0 + rc) / p.div);
-      // Everything this thread needs from global memory is requested BEFORE it waits for the accumulators: its half of
-      // its key's cached half k_t (Wk - Wd) (8 x 128-bit) and, through shared memory, the tile's two query rows.
-      // (ncu, round 1: with the loads inside the j loop the FMA tail sat on the long scoreboard -- 16 dependent L2 round
-      // trips per tile.)
-      const float4* kp = reinterpret_cast<const float4*>(S.Kp + kq_index(ci, S_N / 4, j0 / 4, S_KEYS, key));   // quad jq at kp[jq * 64]
-      float4 kk[S_N / 8];
-#pragma unroll
-      for (int j = 0; j < S_N / 8; ++j) kk[j] = __ldg(kp + j * S_KEYS);
-      if (jh == 0) qa_s[s][e] = __ldg(S.qa + (size_t)rc * S_N + key);
-      named_bar_sync(2, S_EPI_WARPS * 32);         // epilogue warps only; buffer s is rewritten two tiles later
-      mbar_wait(&bar_tfull[s], ph);
-      tc_fence_after();
-      float z[S_N / 2];
-      const uint32_t tl = tbase + ((uint32_t)(ew * 32) << 16);
-#pragma unroll
-      for (int c = 0; c < S_N / 2; c += 16) tmem_ld16(tl + s * S_N + j0 + c, z + c);
-      tmem_wait_ld();
-      tc_fence_before();
-      mbar_arrive(&bar_tempty[s]);               // accumulators are free again
-      const float* qap = qa_s[s] + rr * S_N + j0;
-      // second layer 64 -> 16 as packed fp32 FMAs (fma.rn.f32x2 = SASS FFMA2: two independent fp32 FMAs per issue slot, same
-      // rounding as the scalar form): the kernel is issue-bound on these 512 FMAs + 128 LDS per thread and tile
-      float2 o2[8];
-#pragma unroll
-      for (int jj = 0; jj < 8; ++jj) o2[jj] = jh ? make_float2(0.f, 0.f) : make_float2(b2_s[2 * jj], b2_s[2 * jj + 1]);
-#pragma unroll
-      for (int j = 0; j < S_N / 2; j += 4) {
-        const float4 kq = kk[j / 4];
-        const float4 qq = *reinterpret_cast<const float4*>(qap + j);
-        float zz[4] = {z[j] + qq.x + kq.x, z[j + 1] + qq.y + kq.y, z[j + 2] + qq.z + kq.z, z[j + 3] + qq.w + kq.w};
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const float a1 = fast_sigmoid(zz[u]);  // ex2.approx + rcp.approx (2^-22 / 1 ulp), as in the AUGRU gates
-          const float2 aa = make_float2(a1, a1);
-          const float4* wrow = reinterpret_cast<const float4*>(W2_s + (j0 + j + u) * 16);
-#pragma unroll
-          for (int q4 = 0; q4 < 4; ++q4) {
-            const float4 ww = wrow[q4];
-            ffma2(o2[2 * q4], aa, make_float2(ww.x, ww.y));
-            ffma2(o2[2 * q4 + 1], aa, make_float2(ww.z, ww.w));
-          }
-        }
-      }
-      float o[16];
-#pragma unroll
-      for (int jj = 0; jj < 8; ++jj) { o[2 * jj] = o2[jj].x; o[2 * jj + 1] = o2[jj].y; }
-      // pair hand-over: buffer s of the partial-sum columns is rewritten two tiles later, after the partner's read of it
-      // (the partner reads before it arrives at the next tile's pair barrier, which the writer also passes)
-      const uint32_t tpart = tl + S_TC_PART + s * 16;
-      if (jh) { tmem_st16(tpart, o); tmem_wait_st(); tc_fence_before(); }
-      named_bar_sync(4 + ew, 64);
-      if (!jh) {
-        float o2[16];
-        tc_fence_after();
-        tmem_ld16(tpart, o2);
-        tmem_wait_ld();
-        float sc = S.bk;
-#pragma unroll
-        for (int jj = 0; jj < 16; ++jj) sc = fmaf(fast_sigmoid(o[jj] + o2[jj]), kv_s[jj], sc);
-        if (r < p.R) S.scoresT[((size_t)(r >> 7) * S_KEYS + key) * 128 + (r & 127)] = sc;
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == S_W_MMA) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tbase), "r"(256));
-}
-
 // ------------------------------------------------------------------------------------------------
-// k_scores_tc2 -- the same scores with the SECOND attention layer (64 -> 16) on the tensor pipe as well.
+// k_scores_tc2 -- both attention layers on the tensor pipe.
 //
-// ncu on k_scores_tc (round 2, profiles/r02_k_scores_tc_ncu.txt): 4.5 warps per scheduler, 11.6 cycles per issued
-// instruction, the largest stall the shared-memory scoreboard -- each epilogue warp is ONE dependency chain of ~800
-// instructions per tile (256 FFMA2 + 128 LDS.128 of W2 rows + 32 sigmoids), and that chain, not HBM, sets the tile period.
-// Here the epilogue threads only produce z1 = sigmoid(first layer) and hand it to the MMA warp as the A operand of a
-// second GEMM  [128 rows x 64] x [64 x 16]:
+// Layer 1: the only GEMM-shaped term, (q*k_t) Wp, is a [64 keys x 128] x [128 x 64] product per (row, sequence).  Two
+// feature rows are stacked into one UMMA tile (M = 128 key rows, N = 64, K = 128).  Persistent CTAs loop over tiles;
+// producer warps build A = q*H as bf16 hi/lo core matrices in shared memory (double buffered), one lane issues 5 MMAs per
+// K16 slice (A hi/lo x Wp hi/mid/lo: 2-way x 3-way split, smallest products first), fp32 accumulation in TMEM.
+// Layer 2 (64 -> 16) is a second GEMM  [128 rows x 64] x [64 x 16]  instead of FMAs in the epilogue.  With the FMA form
+// each epilogue warp was ONE dependency chain of ~800 instructions per tile (256 FFMA2 + 128 LDS.128 of W2 rows + 32
+// sigmoids; ncu, round 2, profiles/r02_k_scores_tc_ncu.txt: 11.6 cycles per issued instruction, the largest stall the
+// shared-memory scoreboard), and that chain, not HBM, set the tile period: 158.8 us per 4096-row pass against 90.8 us
+// for this form.  The epilogue threads only produce z1 = sigmoid(first layer) and hand it to the MMA warp:
 //   * A operand IN TENSOR MEMORY (tcgen05.mma ... [d], [a], b-desc: lane = row, 32-bit column c of a K16 slice = the bf16
-//     pair (k = 2c, 2c + 1); layout confirmed by tools/ts_probe.cu): a thread packs its 32 activations as bf16 hi / lo
-//     pairs and writes them with two tcgen05.st into its own TMEM lane -- no shared memory, no proxy fence, and the two
-//     warps of a lane quarter (units 0-31 / 32-63) simply fill different columns, so the round-2 hand-over of partial sums
-//     between them is gone;
+//     pair (k = 2c, 2c + 1); layout confirmed by tools/ts_probe.cu): a thread packs its 16 activations as bf16 hi / lo
+//     pairs and writes them with two tcgen05.st into its own TMEM lane -- no shared memory, no proxy fence, and the four
+//     warps of a lane quarter (16 hidden units each) simply fill different columns;
 //   * B operand = W2 as bf16 hi / mid / lo K-major core matrices (6 KB, appended to the Wp image), 5 MMAs per K16 slice in
-//     the order of the first layer (smallest products first): same 2-way x 3-way split, fp32 accumulation in TMEM;
+//     the order of the first layer: same 2-way x 3-way split, fp32 accumulation in TMEM;
 //   * the second-layer tail (16 sigmoids . kv) of tile i runs after the thread has produced z1 of tile i + 1, so nobody
 //     waits for the MMA warp in steady state; the MMA warp issues layer 1 of tile i + 1 before layer 2 of tile i.
 // Loads roll one tile ahead in both roles: a register that has been consumed is refilled with the next tile's value at
@@ -411,12 +195,6 @@ constexpr int S2_PROD_WARPS = 8, S2_EPI_WARPS = 16;          // 16 epilogue warp
 constexpr int S2_W_MMA = S2_PROD_WARPS + S2_EPI_WARPS, S2_W_LOAD = S2_W_MMA + 1;
 constexpr int S2_THREADS = (S2_W_LOAD + 1) * 32;               // 832: 7 warps on the fullest scheduler -> 72 registers per thread
 
-__device__ __forceinline__ uint32_t elect_one_s() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .b32 r;\n\t.reg .pred p;\n\telect.sync r|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}\n" : "=r"(pred));
-  return pred;
-}
-
 // DBG (tools/scores_probe.cu only): dbg[0..15] = cycles CTA (0, 0) spent per role and phase, summed over its tiles:
 //   producer thread 0:  [0] bar.sync (q rows)  [1] wait A stage free  [2] convert + store
 //   MMA leader:         [4] wait A full  [5] wait accumulators free  [6] issue layer 1  [7] wait A2 full  [8] issue layer 2
@@ -435,7 +213,7 @@ __host__ __device__ inline int scores_grid_split(int ctas, int ntiles, int share
   return n0;
 }
 
-template <bool DBG, bool PF_L2 = false>
+template <bool DBG>
 __global__ void __launch_bounds__(S2_THREADS, 1) k_scores_tc2(ScoreTcParams p, int n0, long long* dbg = nullptr) {
   // 1-D grid: CTAs [0, n0) walk the tiles of sequence 0, CTAs [n0, gridDim.x) those of sequence 1 (scores_grid_split)
   const int sq = (int)blockIdx.x >= n0 ? 1 : 0;
@@ -483,7 +261,7 @@ __global__ void __launch_bounds__(S2_THREADS, 1) k_scores_tc2(ScoreTcParams p, i
   } else if (warp == S2_W_MMA) {
     // ===== MMA issuer: the whole warp walks the tiles in uniform control flow, one elected lane issues (the
     // `if (lane == 0)` form wraps every tcgen05.mma in an ELECT / BRA.U.ANY convergence loop: r4_augru_pair2.cuh) =====
-    const uint32_t leader = elect_one_s();
+    const uint32_t leader = elect_one();
     constexpr uint32_t idesc = make_idesc(TM, S_N), idesc2 = make_idesc(TM, AH2_N);
     mbar_wait(&bar_w, 0);
     const uint32_t b0 = smem_u32(sB), w0 = b0 + S_B_BYTES;
@@ -549,10 +327,12 @@ __global__ void __launch_bounds__(S2_THREADS, 1) k_scores_tc2(ScoreTcParams p, i
   } else if (warp < S2_PROD_WARPS) {
     // ===== producers: A = q * H as bf16 hi/lo.  Load g = 0..15 of a thread: K block kb = g % 4, row group g / 4; a warp reads
     // 4 rows x 128 contiguous bytes per 128-bit load (lane = row lane / 8, 16-byte piece lane % 8): whole lines, 4 L1
-    // wavefronts per warp load (k_scores_tc's (row, 32-byte chunk) mapping read half of every sector per load: 8 wavefronts).
+    // wavefronts per warp load (a (row, 32-byte chunk) mapping reads half of every sector per load: 8 wavefronts).
     // A thread therefore owns HALF a core-matrix row (4 of its 8 K values) and stores it with one 64-bit store per split; with
     // the 160-byte K stride the 32 half rows of a warp store (4 rows x 4 chunks x 2 halves) cover every bank exactly twice.
     // Eight loads are in flight per thread: load g + 8 is issued into the register load g has just been consumed from.
+    // (Pulling the next tile's lines into L2 a tile period early measured 90.1 against 90.3 us per pass: the producers of
+    // an HBM-fed sequence are capped by what one SM's L1 keeps in flight, 11.5 B/clk, not by DRAM latency.)
     const int prow = warp * 4 + (lane >> 3), piece = lane & 7;
     // the 16 loads of a tile are constant offsets from two row bases (feature rows 2 tile, 2 tile + 1): g / 8 picks the
     // feature row, (g / 4) % 2 the upper 32 keys, g % 4 the K block
@@ -592,20 +372,6 @@ __global__ void __launch_bounds__(S2_THREADS, 1) k_scores_tc2(ScoreTcParams p, i
       uint8_t* a = sA + s * S_A_STAGE;
       const float* h1 = hbase(tile, 1);            // second feature row of this tile (loads 8..15)
       const float* hn = hbase(more ? tn : tile, 0);   // first feature row of the next tile
-      // Probe switch (tools/scores_probe.cu): one lane per 128-byte line pulls the next lines of H into L2 a tile period early.
-      // Measured: 90.1 us with, 90.3 us without -- the producers of an HBM-fed sequence are not waiting for DRAM latency
-      // (the loads of a CTA are capped by what one SM's L1 keeps in flight: 11.5 B/clk here against 65 B/clk for bulk
-      // copies, r02_l2_ingest_probe); kept off in the product build.
-      if (PF_L2 && piece == 0 && !S.shared) {
-        const int t2 = tn + nbx;
-        const float* pa = more ? hbase(tn, 1) : nullptr;
-        const float* pb = t2 < ntiles ? hbase(t2, 0) : nullptr;
-#pragma unroll
-        for (int g = 0; g < 8; ++g) {
-          if (pa) asm volatile("prefetch.global.L2 [%0];" :: "l"(pa + hoff(g + 8)));
-          if (pb) asm volatile("prefetch.global.L2 [%0];" :: "l"(pb + hoff(g)));
-        }
-      }
 #pragma unroll
       for (int g = 0; g < 16; ++g) {
         const int m = (g >> 2) * 32 + prow;
@@ -629,8 +395,7 @@ __global__ void __launch_bounds__(S2_THREADS, 1) k_scores_tc2(ScoreTcParams p, i
   } else if (warp < S2_W_MMA) {
     // ===== epilogue: lane = key row of the tile; the four warps of a TMEM lane quarter take 16 hidden units of the first
     // attention layer each (jq = 0..3) and write their columns of the second GEMM's A operand; the 16-wide tail of tile i is
-    // run, one tile behind, by column quarter i % 4.  (k_scores_tc: 8 epilogue warps with 32 units each -- ncu: 11.6 cycles
-    // per issued instruction and warp, ~800 instructions per warp and tile: that one chain WAS the tile period.) =====
+    // run, one tile behind, by column quarter i % 4. =====
     const int e = (tid - S2_PROD_WARPS * 32) & 127;  // row of the tile: 0..127
     const int jq = (tid - S2_PROD_WARPS * 32) >> 7;  // column quarter
     const int ew = e >> 5;                       // TMEM lane quarter (= warp % 4)

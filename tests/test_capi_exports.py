@@ -118,27 +118,30 @@ def test_c99_caller_compiles_links_and_runs(tmp_path):
     assert "sizeof r4_config %d r4_out %d" % (C.sizeof(_capi.R4Config), C.sizeof(_capi.R4Out)) in out
 
 
-def test_set_option_accepts_what_the_header_documents():
-    """r4_set_option: every key the header lists is accepted with a documented value and restored; unknown keys and
-    out-of-range values are R4_ERR_ARG with a message (no GPU involved: process-wide host state)."""
+def test_set_option_accepts_the_documented_keys_and_rejects_removed_ones():
+    """r4_set_option: every key the header lists is accepted with a documented value and restored; the keys of the
+    removed kernel variants, unknown keys and out-of-range values are R4_ERR_ARG with a message (no GPU involved:
+    process-wide host state)."""
     lib = _capi.load_library()
     text = open(os.path.join(ROOT, "include", "rl4rs_b200.h")).read()
     block = text[text.index("Process-wide kernel-choice overrides"):text.index("int r4_set_option")]
     keys = set(re.findall(r'"([a-z_0-9]+)"', block))
-    defaults = {"augru_kernel": 0, "augru_pair_impl": 1, "augru_cost_pair": 13, "augru_cost_pp": 24, "augru_cluster": 2,
-                "pay_obs_reuse": 1, "scores_impl": 2, "scores_shared_pct": 85}
+    defaults = {"augru_kernel": 0, "augru_cost_pair": 13, "augru_cost_pp": 24, "pay_obs_reuse": 1, "scores_shared_pct": 85}
     assert keys == set(defaults), keys ^ set(defaults)
     try:
-        for k, other in (("augru_kernel", 3), ("augru_pair_impl", 4), ("augru_cost_pair", 7), ("augru_cost_pp", 9),
-                         ("augru_cluster", 8), ("pay_obs_reuse", 0), ("scores_impl", 1), ("scores_shared_pct", 50)):
+        for k, other in (("augru_kernel", 3), ("augru_cost_pair", 7), ("augru_cost_pp", 9), ("pay_obs_reuse", 0),
+                         ("scores_shared_pct", 50)):
             assert lib.r4_set_option(k.encode(), other) == 0, k
         # the rule reads the costs just set (7 : 9): one wave of 64 tile-sequences -> pair; 8 waves against 4 -> ping-pong
         assert lib.r4_augru_kernel_for(64, 148) == 2 and lib.r4_augru_kernel_for(592, 148) == 3
     finally:
         for k, v in defaults.items():
             assert lib.r4_set_option(k.encode(), v) == 0, k
+    # the kernel variants these keys used to select are gone, and so are the keys
+    for k, v in (("augru_pair_impl", 1), ("augru_cluster", 2), ("scores_impl", 2)):
+        assert lib.r4_set_option(k.encode(), v) == -1 and k.encode() in lib.r4_last_error(None), k
     assert lib.r4_set_option(b"no_such_option", 1) == -1 and b"no_such_option" in lib.r4_last_error(None)
-    assert lib.r4_set_option(b"augru_cluster", 3) == -1 and lib.r4_set_option(b"scores_shared_pct", 5) == -1
+    assert lib.r4_set_option(b"augru_kernel", 1) == -1 and lib.r4_set_option(b"scores_shared_pct", 5) == -1
 
 
 def test_host_only_entry_points_agree_with_the_python_side():

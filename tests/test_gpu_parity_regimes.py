@@ -5,8 +5,8 @@
 * full-size batches (4096 and 8192 rows per GPU, the BASELINE configs[1] / north-star per-GPU sizes): a 128-row oracle
   sample of the big env, rows compared by index;
 * every AUGRU kernel forced in turn (``r4_set_option('augru_kernel', ...)``): the simulator alone and env fixtures
-  through the pair kernel (one recurrence per CTA pair) and the ping-pong kernel (two per pair), every hand-over /
-  weight-ring variant of both, plus a launch big enough for the natural rule;
+  through the pair kernel (one recurrence per CTA pair) and the ping-pong kernel (two per pair), plus a launch big
+  enough for the natural rule;
 * the chunked sequence-cache build (> 8192 sequences) and the multi-wave persistent GEMM (tiles > SMs).
 
 Oracle = oracle/env_np.py + oracle/dien_np.py (f32), reference lines: rl4rs/nets/utils.py:117-125,
@@ -151,27 +151,6 @@ def test_dien_forward_each_augru_kernel(kernel, regime, augru_option):
     o_ref, p_ref = DienOracle(w, np.float32).forward(seq, dense, catf)
     assert_close_rel(obs.cpu().numpy(), o_ref, what="dien obs [%s, %s]" % (kernel, regime))
     assert_close_rel(probs.cpu().numpy(), p_ref, what="dien probs [%s, %s]" % (kernel, regime))
-
-
-@pytest.mark.parametrize("impl", [2, 3, 4])
-@pytest.mark.parametrize("kernel", ["pair", "pp"])
-def test_dien_forward_each_pair_variant(kernel, impl, augru_option):
-    """The non-default hand-over / weight-ring variants of the pair kernels (r4_set_option('augru_pair_impl', 2..4):
-    tensor-map ring, relayed release.cluster hand-over, both) against the oracle; 300 rows = 3 tiles, a padding pair."""
-    from oracle.dien_np import DienOracle
-    from rl4rs_b200 import _capi
-    cfg, cat, log, w = _default_regime(8, False)
-    env = make_env(cfg, False, cat, log, w, output_format="numpy")
-    seq, dense, catf = _random_feature_rows(300, 9, 100000)
-    augru_option(kernel)
-    try:
-        _capi.set_option("augru_pair_impl", impl)
-        obs, probs = env.sim.engine.dien_forward(seq, dense, catf)
-    finally:
-        _capi.set_option("augru_pair_impl", 1)
-    o_ref, p_ref = DienOracle(w, np.float32).forward(seq, dense, catf)
-    assert_close_rel(obs.cpu().numpy(), o_ref, what="dien obs [%s, impl %d]" % (kernel, impl))
-    assert_close_rel(probs.cpu().numpy(), p_ref, what="dien probs [%s, impl %d]" % (kernel, impl))
 
 
 @pytest.mark.parametrize("kernel", ["pair", "pp"])

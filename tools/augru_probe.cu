@@ -1,41 +1,17 @@
-// augru_probe.cu -- standalone check + timing of the AUGRU pair kernels (-DPAIR: k_augru_pair2, -DPAIR -DPP: k_augru_pp)
+// augru_probe.cu -- standalone check + timing of the AUGRU pair kernels (default: k_augru_pair2, -DPP: k_augru_pp)
 // against a CPU (f64) recurrence.
 // Build: nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo -o tools/build/augru_probe tools/augru_probe.cu
-#include "../rl4rs_b200/csrc/r4_augru_tc.cuh"
-#ifdef PAIR
-#include "../rl4rs_b200/csrc/r4_augru_pair.cuh"
-#ifndef PAIR2
-#define PAIR2            // the first-generation pair kernel is gone: -DPAIR means k_augru_pair2
-#endif
-#ifdef PAIR2
-#include "../rl4rs_b200/csrc/r4_augru_pair2.cuh"
-#ifndef P2RELAY
-#define P2RELAY R4P2_RELAY
-#endif
-#ifndef P2TMAP
-#define P2TMAP R4P2_TMAP
-#endif
-#ifdef PP
 #include "../rl4rs_b200/csrc/r4_augru_pp.cuh"
-#define KERNEL (k_augru_pp<P2RELAY>)
-#else
-#ifndef P2CS
-#define P2CS 2
-#endif
-#define KERNEL (k_augru_pair2<P2RELAY, P2TMAP, P2CS>)
-#define CLUSTER P2CS
-#endif
-#endif
 #ifdef PP
+#define KERNEL k_augru_pp
 #define KSMEM PP_SMEM_BYTES
 #else
+#define KERNEL k_augru_pair2
 #define KSMEM P_SMEM_BYTES
+#define CLUSTER 2
 #endif
 #define KTHREADS NTHREADS
 #define GRIDX(t) (2 * (t))
-#else
-#error "build with -DPAIR (k_augru_pair2) or -DPAIR -DPP (k_augru_pp): the one-CTA kernel was deleted at the end of round 2"
-#endif
 #include <cstdio>
 #include <cstdlib>
 #include <cmath>
@@ -45,8 +21,6 @@ using namespace r4tc;
 #define CK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { printf("CUDA error %s at %s:%d\n", cudaGetErrorString(e_), __FILE__, __LINE__); exit(1); } } while (0)
 
 static float frand(float a) { return a * ((rand() % 20001) - 10000) / 10000.f; }
-static uint16_t bf16_bits(float x) { uint32_t u; memcpy(&u, &x, 4); u = (u + 0x7fff + ((u >> 16) & 1)) >> 16; return (uint16_t)u; }
-static float bf16_val(uint16_t b) { uint32_t u = (uint32_t)b << 16; float f; memcpy(&f, &u, 4); return f; }
 
 void build_image(const std::vector<float>& Wg, const std::vector<float>& Wc, std::vector<uint8_t>& img) {
   img.assign(W_IMAGE_BYTES, 0);
@@ -67,13 +41,8 @@ int main(int argc, char** argv) {
   for (auto& s : sc) s = 0.5f + frand(0.5f);
   int ctiles = (ncache + TM - 1) / TM, rtiles = (R + TM - 1) / TM;
   std::vector<float> XT((size_t)ctiles * 64 * 768 * TM, 0.f), sT((size_t)rtiles * 64 * TM, 0.f);
-#if defined(PAIR2) && R4P2_PRESCALE
-#define XSCALE(col) ((col) < 512 ? -1.4426950408889634f : 2.8853900817779268f)
-#else
-#define XSCALE(col) 1.0f
-#endif
   for (int c = 0; c < ncache; ++c) for (int t = 0; t < 64; ++t) for (int col = 0; col < 768; ++col)
-    XT[(((size_t)(c / TM) * 64 + t) * 768 + (col & ~3)) * TM + (c % TM) * 4 + (col & 3)] = XSCALE(col) * X[((size_t)c * 64 + t) * 768 + col];   // quad layout (r4_gemm_tc.cuh: xt_index)
+    XT[(((size_t)(c / TM) * 64 + t) * 768 + (col & ~3)) * TM + (c % TM) * 4 + (col & 3)] = X[((size_t)c * 64 + t) * 768 + col];   // quad layout (r4_gemm_tc.cuh: xt_index)
   for (int r = 0; r < R; ++r) for (int t = 0; t < 64; ++t) sT[((size_t)(r / TM) * 64 + t) * TM + r % TM] = sc[(size_t)r * 64 + t];
   std::vector<uint8_t> img; build_image(Wg, Wc, img);
   // CPU reference (f64)
@@ -97,7 +66,6 @@ int main(int argc, char** argv) {
   CK(cudaMemcpy(dimg, img.data(), img.size(), cudaMemcpyHostToDevice));
   CK(cudaMemset(dout, 0, (size_t)R * 256 * 4));
   CK(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, KSMEM));
-#ifdef PAIR2
   CUtensorMap tmap;
   { int trc = make_pair_tensor_map(dimg, &tmap); if (trc) { printf("make_pair_tensor_map failed: %d\n", trc); return 1; } }
 #ifdef CLUSTER
@@ -108,9 +76,6 @@ int main(int argc, char** argv) {
     CK(cudaLaunchKernelEx(&lc_, KERNEL, pp_)); } while (0)
 #else
 #define LAUNCH(grid, prm) do { AugruPairParams pp_; pp_.b = (prm); pp_.tmap[0] = tmap; pp_.tmap[1] = tmap; KERNEL<<<grid, KTHREADS, KSMEM>>>(pp_); } while (0)
-#endif
-#else
-#define LAUNCH(grid, prm) KERNEL<<<grid, KTHREADS, KSMEM>>>(prm)
 #endif
   AugruTcParams p{};
   p.s[0] = {dXT, dimg, dsT, dout, 0}; p.s[1] = p.s[0];
@@ -168,7 +133,7 @@ int main(int argc, char** argv) {
 #endif
       if (it == 2) {
         long long hd[64 * 16]; CK(cudaMemcpy(hd, ddbg, sizeof(hd), cudaMemcpyDeviceToHost));
-#ifdef PAIR
+#ifndef PP
         for (int t = 10; t < 13; ++t) {
           long long* d = hd + t * 16;
           printf("  step %d MMA thread: wait h %lld | issue r %lld | issue u %lld | wait rh %lld | issue c %lld | total %lld (waits: operand quarters %lld, ring stages %lld)\n", t, d[1] - d[0],

@@ -1,7 +1,7 @@
-// scores_probe.cu -- k_scores_tc (second attention layer as FFMA2 in the epilogue) against k_scores_tc2 (second layer as a
-// tcgen05 GEMM with the A operand in tensor memory): both checked against an f64 CPU evaluation of
+// scores_probe.cu -- k_scores_tc2 checked against an f64 CPU evaluation of
 //   score = sigmoid(sigmoid(qa + Kp + (q * H) Wp) W2 + b2) . kv + bk        (r4_scores_tc.cuh)
-// on random inputs, then timed on an observation-pass-sized launch (sequence 0 unshared, sequence 1 shared, as in Slate).
+// on random inputs, then timed on an observation-pass-sized launch (sequence 0 unshared, sequence 1 shared, as in Slate)
+// for several CTA shares of the shared sequence, and broken down per role and phase by the instrumented build (DBG).
 // Build: nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo -o tools/build/scores_probe tools/scores_probe.cu
 // Run:   tools/build/scores_probe [rows=4096] [check_rows=300] [reps=20]
 #include "../rl4rs_b200/csrc/r4_scores_tc.cuh"
@@ -31,7 +31,7 @@ int main(int argc, char** argv) {
   const float bk[2] = {0.1f, -0.2f};
   const int rt = (R + 127) / 128;
   ScoreTcParams p{};
-  float* out[2][2];
+  float* out[2];
   for (int i = 0; i < 2; ++i) {
     std::vector<uint8_t> img(S_IMG_BYTES);
     build_scores_image2(Wp[i].data(), W2[i].data(), img.data());
@@ -43,31 +43,25 @@ int main(int argc, char** argv) {
         for (int j = 0; j < 64; ++j) Kq[kq_index(n, 16, j / 4, 64, key) + j % 4] = Kh[(n * 64 + key) * 64 + j];
     s.qa = up(i ? qa1 : qa0); s.H = up(i ? H1 : H0); s.Kp = up(Kq); s.WpImg = up(img);
     s.Wqd = nullptr; s.b1 = nullptr; s.W2 = up(W2[i]); s.b2 = up(b2[i]); s.kv = up(kv[i]); s.bk = bk[i]; s.shared = i;
-    for (int k = 0; k < 2; ++k) { CK(cudaMalloc(&out[k][i], (size_t)rt * 64 * 128 * 4)); CK(cudaMemset(out[k][i], 0xff, (size_t)rt * 64 * 128 * 4)); }
+    CK(cudaMalloc(&out[i], (size_t)rt * 64 * 128 * 4)); CK(cudaMemset(out[i], 0xff, (size_t)rt * 64 * 128 * 4));
   }
   p.q = up(q); p.row0 = 0; p.div = 1;
-  CK(cudaFuncSetAttribute(k_scores_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, S_SMEM_BYTES));
   CK(cudaFuncSetAttribute(k_scores_tc2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, S2_SMEM_BYTES));
   CK(cudaFuncSetAttribute(k_scores_tc2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, S2_SMEM_BYTES));
-  auto launch = [&](int which, int rows) {
+  auto launch = [&](int rows) {
     p.R = rows;
-    for (int i = 0; i < 2; ++i) p.s[i].scoresT = out[which][i];
-    const dim3 grid(std::min((rows + 1) / 2, 74), 2);
-    if (which == 0) k_scores_tc<<<grid, S_THREADS, S_SMEM_BYTES>>>(p, nullptr, nullptr);
-    else {
-      const int ctas = std::min(2 * ((rows + 1) / 2), 148);
-      if (pct < 0) k_scores_tc2<false, true><<<ctas, S2_THREADS, S2_SMEM_BYTES>>>(p, scores_grid_split(ctas, (rows + 1) / 2, 0, 1, -pct));
-      else k_scores_tc2<false><<<ctas, S2_THREADS, S2_SMEM_BYTES>>>(p, scores_grid_split(ctas, (rows + 1) / 2, 0, 1, pct));
-    }
+    for (int i = 0; i < 2; ++i) p.s[i].scoresT = out[i];
+    const int ctas = std::min(2 * ((rows + 1) / 2), 148);
+    k_scores_tc2<false><<<ctas, S2_THREADS, S2_SMEM_BYTES>>>(p, scores_grid_split(ctas, (rows + 1) / 2, 0, 1, pct));
   };
   // ---- correctness on RC rows (odd counts exercise the half-filled last tile), then on all R rows for the first / last rows
   int bad_total = 0;
   for (int rows : {RC, 1, R}) {
-    for (int which = 0; which < 2; ++which) { launch(which, rows); CK(cudaGetLastError()); CK(cudaDeviceSynchronize()); }
-    std::vector<float> o[2][2];
-    for (int k = 0; k < 2; ++k) for (int i = 0; i < 2; ++i) { o[k][i].resize((size_t)rt * 64 * 128); CK(cudaMemcpy(o[k][i].data(), out[k][i], o[k][i].size() * 4, cudaMemcpyDeviceToHost)); }
-    double worst[2] = {0, 0}, worst12 = 0;
-    int bad[2] = {0, 0};
+    launch(rows); CK(cudaGetLastError()); CK(cudaDeviceSynchronize());
+    std::vector<float> o[2];
+    for (int i = 0; i < 2; ++i) { o[i].resize((size_t)rt * 64 * 128); CK(cudaMemcpy(o[i].data(), out[i], o[i].size() * 4, cudaMemcpyDeviceToHost)); }
+    double worst = 0;
+    int bad = 0;
     const int step = rows > 600 ? rows / 300 : 1;
     for (int r = 0; r < rows; r += (r + step < rows || r == rows - 1) ? step : (rows - 1 - r)) {
       for (int i = 0; i < 2; ++i)
@@ -86,40 +80,34 @@ int main(int argc, char** argv) {
           double sc = bk[i];
           for (int n = 0; n < 16; ++n) sc += kv[i][n] / (1.0 + exp(-z2[n]));
           const size_t idx = ((size_t)(r >> 7) * 64 + key) * 128 + (r & 127);
-          for (int k = 0; k < 2; ++k) {
-            const double err = fabs((double)o[k][i][idx] - sc);
-            if (!(err <= 2e-5 * (1.0 + fabs(sc)))) ++bad[k];
-            if (err > worst[k] || err != err) worst[k] = err;
-          }
-          worst12 = fmax(worst12, fabs((double)o[0][i][idx] - (double)o[1][i][idx]));
+          const double err = fabs((double)o[i][idx] - sc);
+          if (!(err <= 2e-5 * (1.0 + fabs(sc)))) ++bad;
+          if (err > worst || err != err) worst = err;
         }
       if (r == rows - 1) break;
     }
-    printf("rows %5d: k_scores_tc worst |err| %.3g (%d bad)   k_scores_tc2 worst |err| %.3g (%d bad)   tc vs tc2 %.3g\n",
-           rows, worst[0], bad[0], worst[1], bad[1], worst12);
-    bad_total += bad[0] + bad[1];
+    printf("rows %5d: k_scores_tc2 worst |err| %.3g (%d bad)\n", rows, worst, bad);
+    bad_total += bad;
   }
   printf("%s\n", bad_total ? "FAIL" : "PASS");
   // ---- timing
   cudaEvent_t e0, e1; CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
-  CK((cudaFuncSetAttribute(k_scores_tc2<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, S2_SMEM_BYTES)));
-  for (int cfg = 0; cfg < 8; ++cfg) {
-    const int which = cfg ? 1 : 0;
-    const int pcts[8] = {100, 100, 85, 75, 65, 55, 45, -75};    // negative: WITH the L2 prefetch probe switch
+  for (int cfg = 0; cfg < 6; ++cfg) {
+    const int pcts[6] = {100, 85, 75, 65, 55, 45};
     pct = pcts[cfg];
-    for (int i = 0; i < 3; ++i) launch(which, R);
+    for (int i = 0; i < 3; ++i) launch(R);
     CK(cudaEventRecord(e0));
-    for (int i = 0; i < reps; ++i) launch(which, R);
+    for (int i = 0; i < reps; ++i) launch(R);
     CK(cudaEventRecord(e1)); CK(cudaEventSynchronize(e1));
     float ms; CK(cudaEventElapsedTime(&ms, e0, e1));
-    printf("timing %s (shared-sequence share %3d%%): %.1f us per launch of %d rows (%d tiles per sequence)\n", which ? "k_scores_tc2" : "k_scores_tc ", pct, 1e3 * ms / reps, R, (R + 1) / 2);
+    printf("timing k_scores_tc2 (shared-sequence share %3d%%): %.1f us per launch of %d rows (%d tiles per sequence)\n", pct, 1e3 * ms / reps, R, (R + 1) / 2);
   }
   pct = 100;
   // ---- where the time of a tile goes (CTA (0, 0) = unshared sequence, instrumented build of the kernel)
   {
     long long* dd; CK(cudaMalloc(&dd, 32 * 8)); CK(cudaMemset(dd, 0, 32 * 8));
     p.R = R;
-    for (int i = 0; i < 2; ++i) p.s[i].scoresT = out[1][i];
+    for (int i = 0; i < 2; ++i) p.s[i].scoresT = out[i];
     const int grid = std::min(2 * ((R + 1) / 2), 148), n0 = scores_grid_split(grid, (R + 1) / 2, 0, 1, 100);
     cudaEvent_t a0, a1; CK(cudaEventCreate(&a0)); CK(cudaEventCreate(&a1));
     k_scores_tc2<true><<<grid, S2_THREADS, S2_SMEM_BYTES>>>(p, n0, dd);
